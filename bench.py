@@ -20,6 +20,11 @@ frames already resident in HBM; `e2e` is the same metric through the public API
 timed region); `roofline` describes the dominant kernel (attention, tensor-core bound);
 `cpu_baseline` is the oracle (a port of the reference algorithm with the same ATen CPU kernels)
 timed on this box's host cores on a bounded sample.
+
+`--dump-outputs DIR` also writes the int64 label maps of the last timed step (what the caller of the timed path receives)
+as DIR/labels.npy in float32 (labels_rank<r>.npy per rank on several GPUs), with the batch index of each frame in
+DIR/labels_frames.npy: inputs and weights are seeded,
+so two builds run with the same arguments can be compared map for map.
 """
 from __future__ import annotations
 
@@ -39,6 +44,7 @@ if ROOT not in sys.path:
 METRIC = "frames/sec at 480px ViT-S/8 DINOSeg (n_blocks=3, MLP head, argmax + 480x480 label map)"
 UNIT = "frames/s"
 FALLBACK_PEAKS = {"hbm_gbs": 6650.0, "bf16_tflops": 1590.0, "bf16_tflops_sustained": 1400.0}
+DUMP_BUDGET = 64 << 20     # bytes written by --dump-outputs, all ranks together
 
 
 def parse_args():
@@ -61,7 +67,12 @@ def parse_args():
     ap.add_argument("--stall-limit", type=float, default=0.0,
                     help="seconds after which a run that has not finished is aborted with an error line instead of "
                          "hanging the box (0 = 300 s + 2 s per step)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the label maps of the last timed step to DIR/*.npy (float32; "
+                         f"at most {DUMP_BUDGET >> 20} MB, a fixed sample of frames if the batch is larger)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     world = int(os.environ.get("WORLD_SIZE", "1"))
     args.scaling = "weak"
     if args.global_batch > 0:
@@ -158,6 +169,25 @@ def ncu_attention_traffic():
     return None, None, None
 
 
+def dump_outputs(out_dir, name, labels, budget):
+    """--dump-outputs: the int label maps [B, H, W] of the last timed step -> out_dir/<name>.npy as float32 (exact for class
+    indices), and the batch index of every frame written -> out_dir/<name>_frames.npy (float64).  A batch that does not fit
+    `budget` bytes is cut to a fixed, seeded sample of frames, the same in every run, so that two builds can be compared
+    output for output."""
+    import numpy as np
+    import torch
+    n = int(labels.shape[0])
+    frame_bytes = labels[0].numel() * 4
+    room = budget - 8 * n - 4096                     # the index array and two .npy headers
+    keep = np.arange(n)
+    if n * frame_bytes > room:
+        keep = np.sort(np.random.default_rng(0).choice(n, max(1, room // frame_bytes), replace=False))
+    out = labels[torch.from_numpy(keep).to(labels.device)].to(torch.float32).cpu().numpy()
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, name + ".npy"), out)
+    np.save(os.path.join(out_dir, name + "_frames.npy"), keep.astype(np.float64))
+
+
 # ------------------------------------------------------------------------------------------
 # clocks during the timed region
 # ------------------------------------------------------------------------------------------
@@ -229,7 +259,7 @@ def cpu_forward_timer(args, sd, cfg):
 
     def run(frames):
         lp = O.forward(sd, cfg, frames, frame_chunk=1)
-        O.labels_from_logprobs(lp, frames.shape[0], g)
+        return O.labels_from_logprobs(lp, frames.shape[0], g)[1]
 
     return run, cores, synthetic
 
@@ -268,8 +298,10 @@ def run_reference_arm(args):
             run(frames)
         t0 = time.perf_counter()
         for _ in range(args.steps):
-            run(frames)
+            labels = run(frames)
         dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, "labels", torch.from_numpy(labels), DUMP_BUDGET)
     fps = args.steps / dt
     sample = (f"1 frame per step out of the step's {args.batch}-frame batch ({args.res}px), fp32 torch CPU ops with "
               f"{cores} threads; frames are independent so frames/s does not depend on the sample size")
@@ -551,6 +583,8 @@ def main():
     }
     if kinds is not None:
         out["kernels"] = kinds
+    if args.dump_outputs:                                          # `labels` is still the last timed step's result
+        dump_outputs(args.dump_outputs, "labels" if world == 1 else f"labels_rank{rank}", labels, DUMP_BUDGET // world)
     if world == 1 and not args.no_extra_configs and (args.arch, args.res, args.n_blocks) == ("vit_small", 480, 3):
         del model, frames, labels                                  # free the workspace of the headline workload
         torch.cuda.empty_cache()

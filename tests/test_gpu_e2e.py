@@ -509,6 +509,26 @@ def test_layernorm1_inside_the_qkv_gemm_matches_the_two_kernel_path(variant):
     assert float((low1 == low0).float().mean()) >= 0.99
 
 
+def test_bench_dumps_the_label_maps_of_its_timed_path(tmp_path):
+    """bench.py --dump-outputs: the float32 copy of the int64 label maps of the last timed step, equal to what
+    DINOSeg.infer returns for the bench's seeded weights (seed 0) and frames (seed 1); --steps is the number of timed steps."""
+    import subprocess
+    import sys
+    dump = tmp_path / "dump"
+    p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", "2", "--warmup", "1", "--res", "240",
+                        "--n-blocks", "1", "--batch", "3", "--no-e2e", "--no-cpu-baseline", "--dump-outputs", str(dump)],
+                       capture_output=True, text=True, timeout=600)
+    assert p.returncode == 0, p.stderr[-2000:]
+    r = json.loads([l for l in p.stdout.splitlines() if l.startswith("{")][-1])
+    assert r["steps"] == 2 and r["gpu_launches"] % 2 == 0
+    got = np.load(dump / "labels.npy")
+    assert got.dtype == np.float32 and got.shape == (3, 480, 480)
+    assert np.load(dump / "labels_frames.npy").tolist() == [0.0, 1.0, 2.0]
+    m, cfg, sd = _model("vit_small", 1, 0, "reference_init")
+    _, _, lab = m.infer(synthetic.make_frames(3, 240, seed=1).cuda(), want_logprobs=False, want_labels=True)
+    assert np.array_equal(got, lab.cpu().numpy().astype(np.float32))
+
+
 def test_weight_update_is_picked_up():
     """load_state_dict after the first forward re-packs the bf16 weights (no stale cache)."""
     m, cfg, sd = _model("vit_small", 1, 1, "reference_init")

@@ -216,17 +216,48 @@ def test_two_rank_gloo_sharding(tmp_path):
     assert r["ok"] and r["world"] == 2
 
 
-def test_bench_reference_arm_contract():
-    """`bench.py --impl reference` prints one JSON line with the reference-arm keys (tiny config)."""
+def test_bench_reference_arm_contract(tmp_path):
+    """`bench.py --impl reference` prints one JSON line with the reference-arm keys (tiny config); --dump-outputs writes
+    the label map of its last timed step (frame 0 of the batch)."""
     import json
+    from oracle import dinoseg_oracle as O
+    dump = tmp_path / "dump"
     p = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1",
-                        "--warmup", "1", "--res", "64", "--n-blocks", "1", "--batch", "2"],
+                        "--warmup", "1", "--res", "64", "--n-blocks", "1", "--batch", "2", "--dump-outputs", str(dump)],
                        capture_output=True, text=True, timeout=300)
     assert p.returncode == 0, p.stderr[-2000:]
     r = json.loads([l for l in p.stdout.splitlines() if l.startswith("{")][-1])
     assert r["impl"] == "reference" and r["unit"] == "frames/s" and r["value"] > 0
     assert r["cpu_baseline"]["kind"] == "port" and r["cpu_baseline"]["cores"] >= 1
     assert r["e2e"]["h2d_bytes_per_step"] == 0 and r["e2e"]["value"] == r["value"]
+    got = np.load(dump / "labels.npy")
+    assert got.dtype == np.float32 and got.shape == (1, 480, 480)
+    assert np.load(dump / "labels_frames.npy").tolist() == [0.0]
+    cfg = synthetic.make_config("vit_small", 1, 7)
+    lp = O.forward(synthetic.init_state_dict(cfg, 0, "reference_init"), cfg, synthetic.make_frames(1, 64, seed=1),
+                   frame_chunk=1)
+    assert np.array_equal(got, O.labels_from_logprobs(lp, 1, 8)[1].astype(np.float32))
+
+
+def test_bench_dump_samples_a_fixed_set_of_frames_over_budget(tmp_path):
+    """--dump-outputs keeps under its byte budget: a batch that does not fit is cut to a seeded sample of frames (the same
+    in every run, listed in <name>_frames.npy); a batch that fits is written whole."""
+    import importlib
+    sys.path.insert(0, ROOT)
+    bench = importlib.import_module("bench")
+    labels = torch.arange(10 * 4 * 4, dtype=torch.int64).reshape(10, 4, 4)
+    budget = 4096 + 8 * 10 + 3 * 4 * 4 * 4                       # headers and index + three float32 frames
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), "labels", labels, budget)
+    keep = np.load(tmp_path / "a" / "labels_frames.npy")
+    got = np.load(tmp_path / "a" / "labels.npy")
+    assert keep.dtype == np.float64 and len(keep) == 3 and (np.diff(keep) > 0).all()
+    assert got.dtype == np.float32 and np.array_equal(got, labels.numpy()[keep.astype(int)].astype(np.float32))
+    assert np.array_equal(np.load(tmp_path / "b" / "labels_frames.npy"), keep)
+    assert sum(f.stat().st_size for f in (tmp_path / "a").iterdir()) <= budget
+    bench.dump_outputs(str(tmp_path / "c"), "labels", labels, 1 << 20)
+    assert np.array_equal(np.load(tmp_path / "c" / "labels.npy"), labels.numpy().astype(np.float32))
+    assert np.load(tmp_path / "c" / "labels_frames.npy").tolist() == list(range(10))
 
 
 @pytest.mark.parametrize("g,p,offset", [(60, 8, 0), (30, 16, 0), (62, 7, 0), (3, 160, 0), (1, 480, 0), (5, 96, 8)])
