@@ -75,7 +75,6 @@ SIGNATURES = {
     "dinoseg_set_pair_kernels": (C.c_int, [C.c_void_p, C.c_int]),
     "dinoseg_debug_host_pool": (C.c_int, [C.c_int, C.c_int]),
     "dinoseg_debug_attn_redone": (C.c_int, []),
-    "dinoseg_op_gemm_pair_ln": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_float, C.c_float, C.c_int, C.c_void_p]),
     "dinoseg_debug_attn_items": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_int]),
     "dinoseg_expand_labels_host": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "dinoseg_get_pair_kernels": (C.c_int, [C.c_void_p]),
@@ -84,7 +83,6 @@ SIGNATURES = {
     "dinoseg_half_counts": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]),
     "dinoseg_set_fused_mlp": (C.c_int, [C.c_void_p, C.c_int]),
     "dinoseg_set_fused_head": (C.c_int, [C.c_void_p, C.c_int]),
-    "dinoseg_set_fuse_ln1": (C.c_int, [C.c_void_p, C.c_int]),
     "dinoseg_op_layernorm": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
                                        C.c_float, C.c_void_p]),
     "dinoseg_op_posembed": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),

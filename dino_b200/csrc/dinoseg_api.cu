@@ -175,11 +175,12 @@ cudaError_t launch_mlp_fused(const CUtensorMap& a, const CUtensorMap& w1, const 
 constexpr int kLinPitch = 16;    // row pitch (floats) of the 'linear' head's logits buffer (n_classes <= 16)
 constexpr int kHeadPart = 256;   // width of each bf16x3 part of relu(layer_1) (head_h1 <= 256, zero padded)
 
-template <int EPI, bool RES_A>
-cudaError_t launch_gemm_tt(const CUtensorMap& a, const CUtensorMap& w, const CUtensorMap& out, const CUtensorMap& add,
-                           const GemmParams& p, int num_sms, cudaStream_t s) {
-  auto kern = gemm_bf16_tn_kernel<EPI, RES_A>;
-  constexpr size_t smem = gemm_smem_bytes(EPI, RES_A);
+// Single-CTA launch: persistent CTAs, A and W tiles streamed through the ring.
+template <int EPI>
+cudaError_t launch_gemm_t(const CUtensorMap& a, const CUtensorMap& w, const CUtensorMap& out, const CUtensorMap& add,
+                          const GemmParams& p, int num_sms, cudaStream_t s) {
+  auto kern = gemm_bf16_tn_kernel<EPI, false>;
+  constexpr size_t smem = gemm_smem_bytes(EPI, false, false);
   static_assert(smem <= 227 * 1024, "shared memory budget");
   static bool attr[64] = {};
   int dev = 0;
@@ -193,8 +194,7 @@ cudaError_t launch_gemm_tt(const CUtensorMap& a, const CUtensorMap& w, const CUt
   const int m_tiles = (p.rows_per_batch + GEMM_BM - 1) / GEMM_BM * p.batches;
   const long long total = (long long)n_tiles * m_tiles;
   if (total <= 0 || total > INT32_MAX || p.K % GEMM_BK != 0 || n_tiles * GEMM_BN > GEMM_MAX_N) return cudaErrorInvalidValue;
-  const long long units = RES_A ? m_tiles : total;            // RES_A: CTAs walk whole row blocks
-  const int grid = units < num_sms ? int(units) : num_sms;    // persistent: one CTA per SM
+  const int grid = total < num_sms ? int(total) : num_sms;    // persistent: one CTA per SM
   GemmParams pp = p;
   pp.timing = g_attn_timing;
   pp.hb = g_heartbeat;
@@ -239,71 +239,14 @@ cudaError_t launch_gemm_pair_t(const CUtensorMap& a, const CUtensorMap& w, const
   return cudaLaunchKernelEx(&cfg, kern, a, w, out, add, pp);
 }
 
-// CTA-pair GEMM with the LayerNorm of fp32 rows as its A operand (gemm.cuh, LN_A): K = 384, resident A produced in place.
-// `w` (96-row boxes) and p.bias must carry the LayerNorm's gamma / beta (fold_ln_weight_kernel).
-template <int EPI>
-cudaError_t launch_gemm_pair_ln(const float* x, float eps, const CUtensorMap& w, const CUtensorMap& out, const GemmParams& p,
-                                int num_sms, cudaStream_t s) {
-  auto kern = gemm_bf16_tn_kernel<EPI, true, true, true>;
-  constexpr size_t smem = gemm_smem_bytes(EPI, true, true);
-  static bool attr[64] = {};
-  int dev = 0;
-  cudaGetDevice(&dev);
-  if (!attr[dev & 63]) {
-    cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem));
-    if (e != cudaSuccess) return e;
-    attr[dev & 63] = true;
-  }
-  const int n_tiles = (p.N + GEMM_BN - 1) / GEMM_BN;
-  const int m_tiles = (p.rows_per_batch + GEMM_BM - 1) / GEMM_BM;
-  const long long units = (m_tiles + 1) / 2;
-  if (x == nullptr || units <= 0 || p.K != GEMM_RES_KB * GEMM_BK || p.batches != 1 || p.a_wrap != 0 ||
-      n_tiles * GEMM_BN > GEMM_LN_STATS_OFF)
-    return cudaErrorInvalidValue;
-  const int max_pairs = num_sms / 2;
-  GemmParams pp = p;
-  pp.timing = g_attn_timing;
-  pp.hb = g_heartbeat;
-  pp.ln_x = x;
-  pp.ln_eps = eps;
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3(2 * unsigned(units < max_pairs ? units : max_pairs));
-  cfg.blockDim = dim3(GEMM_THREADS + GEMM_LN_THREADS);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = s;
-  cudaLaunchAttribute at[1];
-  at[0].id = cudaLaunchAttributeClusterDimension;
-  at[0].val.clusterDim.x = 2; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
-  cfg.attrs = at;
-  cfg.numAttrs = 1;
-  return cudaLaunchKernelEx(&cfg, kern, w, w, out, out, pp);   // (the A tensor map is not used)
-}
-
 template <int EPI>
 cudaError_t launch_gemm_pair(const CUtensorMap& a, const CUtensorMap& w, const CUtensorMap& out, const CUtensorMap& add,
                              const GemmParams& p, int num_sms, cudaStream_t s) {
   // resident A (K <= 384: ViT-S qkv) measured best inside the whole step (7.56-7.71 k frames/s against 7.51-7.58 k
-  // for streaming pairs and 7.47-7.54 k for single-CTA tiles); DINOSEG_GEMM_PAIR_RESA=0 selects the streaming pairs
-  static const bool res_env = [] { const char* e = getenv("DINOSEG_GEMM_PAIR_RESA"); return e ? atoi(e) != 0 : true; }();
-  const bool res_a = res_env && p.K <= GEMM_RES_KB * GEMM_BK && p.N > GEMM_BN && p.a_wrap == 0;
+  // for streaming pairs and 7.47-7.54 k for single-CTA tiles)
+  const bool res_a = p.K <= GEMM_RES_KB * GEMM_BK && p.N > GEMM_BN && p.a_wrap == 0;
   return res_a ? launch_gemm_pair_t<EPI, true>(a, w, out, add, p, num_sms, s)
                : launch_gemm_pair_t<EPI, false>(a, w, out, add, p, num_sms, s);
-}
-
-// Single-CTA launches.  The resident-A form (K <= 384, several n-tiles) measured SLOWER than streaming for single
-// CTAs (qkv 0.235 vs 0.200 ms: with the full 24 KB W tiles in the ring the single A buffer cannot be refilled early
-// enough) and is only compiled in with -DDSG_GEMM_RESA; as CTA pairs (12 KB half W tiles, launch_gemm_pair) it is
-// the fastest form and the default for the ViT-S qkv GEMM.
-template <int EPI>
-cudaError_t launch_gemm_t(const CUtensorMap& a, const CUtensorMap& w, const CUtensorMap& out, const CUtensorMap& add,
-                          const GemmParams& p, int num_sms, cudaStream_t s) {
-#ifdef DSG_GEMM_RESA
-  const bool res_a = p.K <= GEMM_RES_KB * GEMM_BK && p.N > GEMM_BN;
-#else
-  const bool res_a = false;
-#endif
-  return res_a ? launch_gemm_tt<EPI, true>(a, w, out, add, p, num_sms, s)
-               : launch_gemm_tt<EPI, false>(a, w, out, add, p, num_sms, s);
 }
 
 cudaError_t launch_gemm(int epi, const CUtensorMap& a, const CUtensorMap& w, const CUtensorMap& out,
@@ -390,10 +333,8 @@ cudaError_t launch_layernorm(const float* x, const float* g, const float* b, __n
   dim3 grid((M + rows_per_block - 1) / rows_per_block);
   if (D == 384 && !split) layernorm384_bf16_kernel<<<(M + 31) / 32, 256, 0, s>>>(x, g, b, y, M, eps);
   else if (D == 768 && !split) layernorm_bf16_kernel<768, false><<<grid, 256, 0, s>>>(x, g, b, y, M, eps);
-  else if (D == 128 && !split) layernorm_bf16_kernel<128, false><<<grid, 256, 0, s>>>(x, g, b, y, M, eps);
   else if (D == 384 && split) layernorm_bf16_kernel<384, true><<<grid, 256, 0, s>>>(x, g, b, y, M, eps);
   else if (D == 768 && split) layernorm_bf16_kernel<768, true><<<grid, 256, 0, s>>>(x, g, b, y, M, eps);
-  else if (D == 128 && split) layernorm_bf16_kernel<128, true><<<grid, 256, 0, s>>>(x, g, b, y, M, eps);
   else return cudaErrorInvalidValue;
   return cudaGetLastError();
 }
@@ -440,11 +381,6 @@ struct BlockW {
   // fc1 as loaded (fp32): fc1_w / fc1_b above are derived from these by finalize_weights - plain bf16 / copy, or with
   // LayerNorm2's gamma / beta folded in when the fused MLP kernel computes the LayerNorm itself
   float *fc1_w32 = nullptr, *fc1_b32 = nullptr;
-  // qkv: the loaded fp32 weight; qkv_w = its bf16 copy; qkv_wf / qkv_bf = with LayerNorm1's gamma / beta folded in, for
-  // the qkv GEMM that computes the LayerNorm itself (launch_gemm_pair_ln)
-  float *qkv_w32 = nullptr, *qkv_bf = nullptr;
-  __nv_bfloat16* qkv_wf = nullptr;
-  CUtensorMap tm_qkv_hf;
   CUtensorMap tm_qkv, tm_proj, tm_fc1, tm_fc2;
   CUtensorMap tm_fc1_g, tm_fc2_g;   // 128-row granule views for the fused MLP kernel
   CUtensorMap tm_fc1_h, tm_fc2_h;   // 64-row half granules (CTA-pair variant)
@@ -612,11 +548,9 @@ struct dinoseg {
   int launches = 0;
   bool fused_mlp = false;           // D = 384 / hidden = 1536: fused fc1 -> GELU -> fc2 kernel
   bool attn_unshifted = true;       // attention without row maxima + the classic kernel as its redo (attention.cuh)
-  bool fuse_ln1 = false;            // ViT-S: LayerNorm1 computed by the qkv GEMM (CTA pairs) instead of its own kernel (opt-in)
-  bool fuse_ln = true;              // ... which also computes LayerNorm2 itself (no LN launch, no bf16 copy of the tokens)
+  bool fuse_ln = true;              // the fused MLP kernel computes LayerNorm2 itself (no LN launch, no bf16 copy of the tokens)
   bool weights_dirty = true;        // fc1_w / fc1_b have to be (re)derived from the loaded parameters
   bool folded = false;              // ... and currently carry LayerNorm2's gamma / beta
-  int reverse_order = 1;            // GEMM / MLP kernels walk the rows last-to-first, LN / attention first-to-last
   // CTA-pair (cta_group::2) kernels: on by default (dinoseg_set_pair_kernels / DINOSEG_PAIR=0 select the single-CTA
   // forms).  Bit-identical results; +2 % on the ViT-S step, +5 % on ViT-B.  A device / partition without 2-CTA
   // clusters makes the launch fail, in which case forward_impl switches to the single-CTA kernels for good.
@@ -820,14 +754,7 @@ int dinoseg_create(const dinoseg_cfg* cfg, int device, dinoseg_t** out) {
     h->mlp_pair = h->fused_mlp && atoi(mode) != 0;
   }
   if (const char* mode = getenv("DINOSEG_HOST_EXPAND")) h->host_expand = atoi(mode) != 0 ? 1 : 0;   // measurement override
-  if (const char* mode = getenv("DINOSEG_REVERSE")) h->reverse_order = atoi(mode) != 0;   // measurement override
   if (const char* mode = getenv("DINOSEG_FUSE_LN")) h->fuse_ln = atoi(mode) != 0;         // measurement override
-  // LayerNorm1 inside the qkv GEMM is OFF by default: measured neutral (LayerNorm 0.086 + qkv 0.181 ms per block against
-  // 0.256-0.265 ms fused).  The fused kernel reads the fp32 rows twice (statistics, then the normalised block) on top of
-  // the W tiles - 834 KB per row block and SM through the ~42 B/clk L2 -> SM path against 540 KB - and turns from
-  // MMA-bound into delivery-bound.  DINOSEG_FUSE_LN1=1 selects it (parity-tested: gemm_ln_* checks).
-  h->fuse_ln1 = false;
-  if (const char* mode = getenv("DINOSEG_FUSE_LN1")) h->fuse_ln1 = cfg->embed_dim == GEMM_RES_KB * GEMM_BK && atoi(mode) != 0;
   if (const char* mode = getenv("DINOSEG_ATTN_UNSHIFTED")) h->attn_unshifted = atoi(mode) != 0;   // measurement override
   if (const char* mode = getenv("DINOSEG_HOST_CHUNK")) h->host_chunk = atoi(mode) > 0 ? atoi(mode) : 0;   // measurement override
   if (const char* mode = getenv("DINOSEG_GEMM_PAIR")) h->gemm_pair = atoi(mode) != 0;   // measurement override
@@ -877,8 +804,6 @@ int dinoseg_create(const dinoseg_cfg* cfg, int device, dinoseg_t** out) {
     rc |= dev_alloc(h, &b.ln1_g, D); rc |= dev_alloc(h, &b.ln1_b, D);
     rc |= dev_alloc(h, &b.ln2_g, D); rc |= dev_alloc(h, &b.ln2_b, D);
     rc |= dev_alloc(h, &b.qkv_w, size_t(3) * D * D); rc |= dev_alloc(h, &b.qkv_b, 3 * D);
-    rc |= dev_alloc(h, &b.qkv_w32, size_t(3) * D * D); rc |= dev_alloc(h, &b.qkv_wf, size_t(3) * D * D);
-    rc |= dev_alloc(h, &b.qkv_bf, 3 * D);
     rc |= dev_alloc(h, &b.proj_w, size_t(D) * D); rc |= dev_alloc(h, &b.proj_b, D);
     rc |= dev_alloc(h, &b.fc1_w, size_t(HID) * D); rc |= dev_alloc(h, &b.fc1_b, HID);
     rc |= dev_alloc(h, &b.fc1_w32, size_t(HID) * D); rc |= dev_alloc(h, &b.fc1_b32, HID);
@@ -886,14 +811,13 @@ int dinoseg_create(const dinoseg_cfg* cfg, int device, dinoseg_t** out) {
     if (rc) break;
     add_slot(h, pre + "norm1.weight", 0, b.ln1_g, {D}); add_slot(h, pre + "norm1.bias", 0, b.ln1_b, {D});
     add_slot(h, pre + "norm2.weight", 0, b.ln2_g, {D}); add_slot(h, pre + "norm2.bias", 0, b.ln2_b, {D});
-    add_slot(h, pre + "attn.qkv.weight", 0, b.qkv_w32, {3 * D, D}); add_slot(h, pre + "attn.qkv.bias", 0, b.qkv_b, {3 * D});
+    add_slot(h, pre + "attn.qkv.weight", 1, b.qkv_w, {3 * D, D}); add_slot(h, pre + "attn.qkv.bias", 0, b.qkv_b, {3 * D});
     add_slot(h, pre + "attn.proj.weight", 1, b.proj_w, {D, D}); add_slot(h, pre + "attn.proj.bias", 0, b.proj_b, {D});
     add_slot(h, pre + "mlp.fc1.weight", 0, b.fc1_w32, {HID, D}); add_slot(h, pre + "mlp.fc1.bias", 0, b.fc1_b32, {HID});
     add_slot(h, pre + "mlp.fc2.weight", 1, b.fc2_w, {D, HID}); add_slot(h, pre + "mlp.fc2.bias", 0, b.fc2_b, {D});
     bool ok = true;
     ok &= make_tmap_2d(&b.tm_qkv, b.qkv_w, 3 * D, D, D, GEMM_BN);
     ok &= make_tmap_2d(&b.tm_qkv_h, b.qkv_w, 3 * D, D, D, GEMM_BN / 2);
-    ok &= make_tmap_2d(&b.tm_qkv_hf, b.qkv_wf, 3 * D, D, D, GEMM_BN / 2);
     ok &= make_tmap_2d(&b.tm_fc1_p, b.fc1_w, HID, D, D, GEMM_BN / 2);
     ok &= make_tmap_2d(&b.tm_fc2_p, b.fc2_w, D, HID, HID, GEMM_BN / 2);
     ok &= make_tmap_2d(&b.tm_proj, b.proj_w, D, D, D, GEMM_BN);
@@ -1129,13 +1053,6 @@ static int finalize_weights(dinoseg_t* h, cudaStream_t s) {
   if (!h->weights_dirty && h->folded == fold) return 0;
   const int D = h->cfg.embed_dim, HID = h->cfg.mlp_hidden;
   for (BlockW& b : h->blocks) {
-    {                                              // qkv: plain bf16 copy, and the form with LayerNorm1 folded in
-      const size_t n = size_t(3) * D * D;
-      f32_to_bf16_kernel<<<unsigned(std::min<size_t>((n + 255) / 256, 4096)), 256, 0, s>>>(b.qkv_w32, b.qkv_w, n);
-      fold_ln_weight_kernel<<<(3 * D * 32 + 255) / 256, 256, 0, s>>>(b.qkv_w32, b.qkv_b, b.ln1_g, b.ln1_b, b.qkv_wf, b.qkv_bf,
-                                                                     3 * D, D);
-      DSG_CUDA(h, cudaGetLastError());
-    }
     if (fold) {
       fold_ln_weight_kernel<<<(HID * 32 + 255) / 256, 256, 0, s>>>(b.fc1_w32, b.fc1_b32, b.ln2_g, b.ln2_b, b.fc1_w, b.fc1_b,
                                                                    HID, D);
@@ -1246,24 +1163,10 @@ static int forward_impl(dinoseg_t* h, WorkBufs& w, const float* frames, const ui
   // ---- transformer blocks (vision_transformer.py:122-140) ----
   for (int i = 0; i < h->cfg.n_blocks; ++i) {
     BlockW& b = h->blocks[i];
-    bool ln1_done = false;
-    if (h->fuse_ln1 && h->gemm_pair) {
-      // LayerNorm1 -> qkv in ONE kernel: the GEMM's extra warps normalise the fp32 tokens straight into its A block
-      GemmParams p = gp(3 * D, D, b.qkv_bf);
-      p.reverse = h->reverse_order ? 0 : 1;      // the producer of x (fc2 epilogue / patch GEMM) wrote it first-to-last
-      p.col_scale = 0.125f * ATT_LOG2E; p.scale_cols = D;
-      LaunchScope ls(h, K_GEMM_QKV, s);
-      if (launch_gemm_pair_ln<EPI_BF16>(w.x, eps, b.tm_qkv_hf, w.tm_qkv_out, p, sms, s) == cudaSuccess) {
-        ln1_done = true; ++n;
-      } else {
-        (void)cudaGetLastError();   // no 2-CTA clusters on this device / partition: LayerNorm kernel + plain GEMM
-        h->fuse_ln1 = false;
-      }
-    }
-    if (!ln1_done) { LaunchScope ls(h, K_LN, s); DSG_CUDA(h, launch_layernorm(w.x, b.ln1_g, b.ln1_b, w.abuf, M, D, eps, false, s)); ++n; }
-    if (!ln1_done) {
+    { LaunchScope ls(h, K_LN, s); DSG_CUDA(h, launch_layernorm(w.x, b.ln1_g, b.ln1_b, w.abuf, M, D, eps, false, s)); ++n; }
+    {
       GemmParams p = gp(3 * D, D, b.qkv_b);
-      p.reverse = h->reverse_order;              // LN1 wrote abuf first-to-last
+      p.reverse = 1;                             // LN1 wrote abuf first-to-last
       p.col_scale = 0.125f * ATT_LOG2E; p.scale_cols = D;  // q * head_dim^-0.5 (vision_transformer.py:73,85), times log2(e): attention.cuh
       LaunchScope ls(h, K_GEMM_QKV, s);
       if (h->gemm_pair &&
@@ -1283,7 +1186,7 @@ static int forward_impl(dinoseg_t* h, WorkBufs& w, const float* frames, const ui
     }
     {
       GemmParams p = gp(D, D, b.proj_b);
-      p.reverse = h->reverse_order;              // the attention kernel wrote abuf first-to-last
+      p.reverse = 1;                             // the attention kernel wrote abuf first-to-last
       LaunchScope ls(h, K_GEMM_PROJ, s);
       DSG_CUDA(h, launch_gemm(EPI_RESID_F32, w.tm_abuf, b.tm_proj, w.tm_x_out, w.tm_x_out, p, sms, s)); ++n;
     }
@@ -1300,7 +1203,7 @@ static int forward_impl(dinoseg_t* h, WorkBufs& w, const float* frames, const ui
       }
       // start with the rows the producer of x / A wrote last: LN2 writes first-to-last (-> walk backwards), the proj GEMM
       // walks backwards itself (-> walk forwards when the LayerNorm is fused and this kernel follows it directly)
-      p.reverse = h->fuse_ln ? (h->reverse_order ? 0 : 1) : h->reverse_order;
+      p.reverse = h->fuse_ln ? 0 : 1;
       LaunchScope ls(h, K_MLP_FUSED, s);
       if (h->mlp_pair && launch_mlp_fused(w.tm_abuf, b.tm_fc1_h, b.tm_fc2_h, w.tm_x_out, p, sms, true, s) != cudaSuccess) {
         (void)cudaGetLastError();   // no 2-CTA clusters on this device / partition: same kernel, one CTA per row block
@@ -1312,7 +1215,7 @@ static int forward_impl(dinoseg_t* h, WorkBufs& w, const float* frames, const ui
       { LaunchScope ls(h, K_LN, s); DSG_CUDA(h, launch_layernorm(w.x, b.ln2_g, b.ln2_b, w.abuf, M, D, eps, false, s)); ++n; }
       {
         GemmParams p = gp(HID, D, b.fc1_b);
-        p.reverse = h->reverse_order;            // LN2 wrote abuf first-to-last; fc2 then reads hid first-to-last
+        p.reverse = 1;                           // LN2 wrote abuf first-to-last; fc2 then reads hid first-to-last
         LaunchScope ls(h, K_GEMM_FC1, s);
         if (h->gemm_pair &&
             launch_gemm_pair<EPI_GELU_BF16>(w.tm_abuf, b.tm_fc1_p, w.tm_hid_out, w.tm_hid_out, p, sms, s) != cudaSuccess) {
@@ -1855,23 +1758,6 @@ int dinoseg_op_gemm_pair(const void* A, const void* W, const float* bias, void* 
   return e == cudaSuccess ? 0 : -3;
 }
 
-int dinoseg_op_gemm_pair_ln(const float* x, const void* W, const float* bias, void* out, int M, int N, float eps,
-                            float col_scale, int scale_cols, void* stream) {
-  if (!x || !W || !out || M <= 0 || N <= 0 || N % 8 != 0) return -1;
-  int dev = 0, sms = 148;
-  cudaGetDevice(&dev);
-  cudaDeviceGetAttribute(&sms, cudaDevAttrMultiProcessorCount, dev);
-  const int K = GEMM_RES_KB * GEMM_BK;
-  CUtensorMap tw, to;
-  GemmParams p{};
-  p.N = N; p.K = K; p.bias = bias; p.col_scale = col_scale; p.scale_cols = scale_cols;
-  p.rows_per_batch = M; p.batches = 1;
-  bool ok = make_tmap_2d(&tw, W, N, K, K, GEMM_BN / 2);
-  ok &= make_tmap_gemm_out(&to, out, false, N, M, 1, N);
-  if (!ok) return -2;
-  return launch_gemm_pair_ln<EPI_BF16>(x, eps, tw, to, p, sms, static_cast<cudaStream_t>(stream)) == cudaSuccess ? 0 : -3;
-}
-
 // Test hook for the worker pool of the host entry points: create a pool of n threads where the creation of thread number
 // fail_at throws (fail_at < 0: none does), run one task per requested thread, destroy the pool.  Returns the number of
 // threads the pool ended up with (0 when not even the first could be created: the caller's DMA fallback), or -1 if the
@@ -1944,13 +1830,6 @@ int dinoseg_set_fused_mlp(dinoseg_t* h, int on) {
   h->fused_mlp = on != 0;
   h->mlp_pair = on == 2;
   h->weights_dirty = true;          // fc1 with / without the folded LayerNorm2
-  return 0;
-}
-
-int dinoseg_set_fuse_ln1(dinoseg_t* h, int on) {
-  if (!h) return -1;
-  if (on && h->cfg.embed_dim != GEMM_RES_KB * GEMM_BK) DSG_FAIL(h, "LayerNorm1 inside the qkv GEMM needs embed_dim 384");
-  h->fuse_ln1 = on != 0;
   return 0;
 }
 

@@ -16,8 +16,8 @@
 //                 -> swizzled shared-memory staging -> TMA store (fully coalesced, tails clipped by
 //                 the tensor map).  Addends (residual stream, positional table) are TMA-loaded into
 //                 the same staging buffers two chunks ahead.
-// RES_A variant (K <= 384): the CTA walks whole 128-row blocks; the A block (all k-blocks, 96 KB) stays
-// resident in shared memory while the CTA sweeps every n-tile of that row block, and is refilled k-block
+// RES_A variant (CTA pairs only, K <= 384): the CTA walks whole 128-row blocks; the A block (all k-blocks, 96 KB)
+// stays resident in shared memory while the pair sweeps every n-tile of its row blocks, and is refilled k-block
 // by k-block during the last n-tile.  Only the W tiles stream through the ring: the plain variant re-reads
 // A and W for every tile and is bound by the L2 -> SM bandwidth (~11-13 TB/s measured), not by the MMAs.
 // All global tensors are described by 3-D tensor maps {cols, rows_per_batch, batches}; plain
@@ -53,11 +53,6 @@ struct GemmParams {
   int a_wrap;           // > 0: A has only a_wrap columns and the k index wraps (bf16x3 operand stored as [hi | lo])
   long long* timing;    // debug (DSG_GEMM_TIMING builds): [grid][3 roles][8] cycle totals
   int* hb;              // diagnostic heartbeat (see hb_mark), may be null
-  // LN_A kernels (fused LayerNorm in front of the GEMM, e.g. norm1 -> qkv, reference vision_transformer.py:117,:133):
-  // A is not loaded; four extra warps produce it as xhat = (x - mean) * rstd from the fp32 rows of ln_x [rows, K = 384]
-  // (gamma / beta live in W and the bias: fold_ln_weight_kernel).
-  const float* ln_x;
-  float ln_eps;
 };
 
 #ifdef DSG_GEMM_TIMING
@@ -76,8 +71,6 @@ constexpr int GEMM_BN = 192;
 constexpr int GEMM_BK = 64;
 constexpr int GEMM_EPI_THREADS = 256;                 // 8 epilogue warps: two per TMEM lane quarter
 constexpr int GEMM_THREADS = 64 + GEMM_EPI_THREADS;
-constexpr int GEMM_LN_THREADS = 128;                  // LN_A kernels: four more warps that produce the A block
-constexpr int GEMM_LN_STATS_OFF = 2048;               // their (mean, rstd) table: floats 2048.. of the bias area (N <= 2048)
 constexpr int GEMM_A_BYTES = GEMM_BM * GEMM_BK * 2;   // 16 KB
 constexpr int GEMM_B_BYTES = GEMM_BN * GEMM_BK * 2;   // 24 KB
 constexpr int GEMM_STAGE_BYTES = GEMM_A_BYTES + GEMM_B_BYTES;
@@ -94,17 +87,15 @@ __host__ __device__ constexpr int gemm_stages(int epi) { return gemm_nbuf(epi) =
 constexpr int GEMM_MAX_N = 3072;                      // bias vector staged in shared memory
 constexpr int GEMM_BIAS_BYTES = GEMM_MAX_N * 4;
 constexpr int GEMM_RES_KB = 6;                        // resident-A variant: up to 6 k-blocks (K <= 384)
-__host__ __device__ constexpr int gemm_res_wstages(int epi) { return gemm_nbuf(epi) == 4 ? 2 : 3; }
 // CTA-pair variant (cta_group::2): a stage holds this CTA's A tile and HALF of the W tile (96 rows)
 constexpr int GEMM_PAIR_STAGE_BYTES = GEMM_A_BYTES + GEMM_B_BYTES / 2;   // 28 KB
 __host__ __device__ constexpr int gemm_pair_stages(int epi) { return gemm_stages(epi) + 1; }
 // ... or, with the A row block resident (K <= 384), only the half W tile (12 KB)
 __host__ __device__ constexpr int gemm_pair_res_wstages(int epi) { return gemm_nbuf(epi) == 4 ? 3 : 6; }
-__host__ __device__ constexpr size_t gemm_smem_bytes(int epi, bool res_a, bool pair = false) {
+__host__ __device__ constexpr size_t gemm_smem_bytes(int epi, bool res_a, bool pair) {
   return (pair ? (res_a ? size_t(GEMM_RES_KB) * GEMM_A_BYTES + size_t(gemm_pair_res_wstages(epi)) * (GEMM_B_BYTES / 2)
                         : size_t(gemm_pair_stages(epi)) * GEMM_PAIR_STAGE_BYTES)
-          : res_a ? size_t(GEMM_RES_KB) * GEMM_A_BYTES + size_t(gemm_res_wstages(epi)) * GEMM_B_BYTES
-                  : size_t(gemm_stages(epi)) * GEMM_STAGE_BYTES) +
+               : size_t(gemm_stages(epi)) * GEMM_STAGE_BYTES) +
          size_t(gemm_nbuf(epi)) * GEMM_STG_BYTES + GEMM_BIAS_BYTES + 1024 /*align*/ + 256;
 }
 
@@ -132,22 +123,20 @@ __device__ __forceinline__ float gelu_erf(float x) {
 // memories.  The plain kernel is bound by the L2 -> SM delivery of its operands (40 KB per k-block per SM at
 // ~42 B/clk/SM against 512 clk of MMA work); the pair loads 28 KB per k-block per SM.  Barriers as in mlp.cuh: what
 // the issuer waits on lives in the leader CTA and collects both CTAs' arrivals, what it signals is multicast.
-// LN_A = true (RES_A kernels with K = 384 only): the resident A block is the LayerNorm of fp32 rows, produced in place by
-// warps 10..13 - statistics while the previous row block is being multiplied, the bf16 block (same K-major
-// SWIZZLE_128B image the TMA load would have left) as soon as the last n-tile's MMAs have released the k-blocks.
-template <int EPI, bool RES_A, bool PAIR = false, bool LN_A = false>
-__global__ void __launch_bounds__(GEMM_THREADS + (LN_A ? GEMM_LN_THREADS : 0), 1)
+template <int EPI, bool RES_A, bool PAIR = false>
+__global__ void __launch_bounds__(GEMM_THREADS, 1)
 gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmW,
                     const __grid_constant__ CUtensorMap tmOut, const __grid_constant__ CUtensorMap tmAdd,
                     const GemmParams p) {
+  // single-CTA resident A measured slower than streaming (qkv 0.235 vs 0.200 ms: with full 24 KB W tiles in the ring
+  // the one A buffer cannot be refilled early enough); the half W tiles of a pair leave room for it
+  static_assert(!RES_A || PAIR, "resident A is a CTA-pair form");
   constexpr bool OUT_F32 = gemm_out_is_f32(EPI);
   constexpr bool HAS_ADD = gemm_has_addend(EPI);
   constexpr bool SPLIT = EPI == EPI_RELU_SPLIT_BF16;
   constexpr int BPC = SPLIT ? 2 : 1;             // staging buffers per chunk
-  constexpr int STAGES = PAIR ? (RES_A ? gemm_pair_res_wstages(EPI) : gemm_pair_stages(EPI))
-                              : (RES_A ? gemm_res_wstages(EPI) : gemm_stages(EPI));
-  constexpr int RING_BYTES = PAIR ? (RES_A ? GEMM_B_BYTES / 2 : GEMM_PAIR_STAGE_BYTES)
-                                  : (RES_A ? GEMM_B_BYTES : GEMM_STAGE_BYTES);
+  constexpr int STAGES = PAIR ? (RES_A ? gemm_pair_res_wstages(EPI) : gemm_pair_stages(EPI)) : gemm_stages(EPI);
+  constexpr int RING_BYTES = PAIR ? (RES_A ? GEMM_B_BYTES / 2 : GEMM_PAIR_STAGE_BYTES) : GEMM_STAGE_BYTES;
   constexpr uint32_t NCTA = PAIR ? 2 : 1;
   constexpr int A_RES_BYTES = RES_A ? GEMM_RES_KB * GEMM_A_BYTES : 0;
   constexpr int NBUF = gemm_nbuf(EPI);
@@ -223,7 +212,7 @@ gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
       mbar_init(&empty_bar[s], 1);
     }
     for (int s = 0; s < GEMM_RES_KB; ++s) {
-      mbar_init(&a_full[s], LN_A ? 4 * NCTA : 1);   // fused LayerNorm: one arrival per producing warp (both CTAs)
+      mbar_init(&a_full[s], 1);
       mbar_init(&a_empty[s], 1);
     }
     for (int s = 0; s < 2; ++s) {
@@ -267,15 +256,10 @@ gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         for (int kb = 0; kb < num_kb; ++kb, ++kc) {
           GEMM_T(7);
           if constexpr (RES_A) {
-            if (nt == 0 && !LN_A) {                // (re)fill the resident A block, k-block by k-block
+            if (nt == 0) {                         // (re)fill the resident A block, k-block by k-block
               mbar_wait(&a_empty[kb], (mi & 1) ^ 1);
-              if constexpr (PAIR) {
-                if (cta_rank == 0) mbar_expect_tx(&a_full[kb], 2 * GEMM_A_BYTES);
-                tma_load_3d_pair(smem + size_t(kb) * GEMM_A_BYTES, &tmA, mapa_rank(&a_full[kb], 0), kb * GEMM_BK, r0, bt);
-              } else {
-                mbar_expect_tx(&a_full[kb], GEMM_A_BYTES);
-                tma_load_3d(smem + size_t(kb) * GEMM_A_BYTES, &tmA, &a_full[kb], kb * GEMM_BK, r0, bt);
-              }
+              if (cta_rank == 0) mbar_expect_tx(&a_full[kb], 2 * GEMM_A_BYTES);
+              tma_load_3d_pair(smem + size_t(kb) * GEMM_A_BYTES, &tmA, mapa_rank(&a_full[kb], 0), kb * GEMM_BK, r0, bt);
             }
           }
           const int s = kc % STAGES;
@@ -295,11 +279,9 @@ gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
                              nt * GEMM_BN + int(cta_rank) * (GEMM_BN / 2));
           } else {
             mbar_expect_tx(&full_bar[s], RING_BYTES);
-            if constexpr (!RES_A) {
-              const int ak = kb * GEMM_BK;
-              tma_load_3d(sr, &tmA, &full_bar[s], (p.a_wrap > 0 && ak >= p.a_wrap) ? ak - p.a_wrap : ak, r0, bt);
-            }
-            tma_load_2d(sr + (RES_A ? 0 : GEMM_A_BYTES), &tmW, &full_bar[s], kb * GEMM_BK, nt * GEMM_BN);
+            const int ak = kb * GEMM_BK;
+            tma_load_3d(sr, &tmA, &full_bar[s], (p.a_wrap > 0 && ak >= p.a_wrap) ? ak - p.a_wrap : ak, r0, bt);
+            tma_load_2d(sr + GEMM_A_BYTES, &tmW, &full_bar[s], kb * GEMM_BK, nt * GEMM_BN);
           }
           GEMM_T(2);
         }
@@ -371,80 +353,6 @@ gemm_bf16_tn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_consta
         commit(&acc_full[as]);
       }
       GEMM_T_DUMP(1);
-    }
-  } else if (LN_A && warp >= 10) {
-    // ---------------- fused LayerNorm: the A block of every row block of this CTA ----------------
-    // As in mlp.cuh: eight lanes per row, four rows per pass; lane `sub` of group `grp` holds float4 number i*8 + sub
-    // of its row, i.e. columns (i*8 + sub)*4 ..+3 -> k-block i/2, 16-byte chunk ((i&1)*8 + sub)/2 of the row's 128
-    // bytes, 8-byte half sub&1.  Rows past the end are written as zeros (what TMA's fill does).
-    if constexpr (LN_A) {
-      const int ow = warp - 10, sub = lane & 7, grp = lane >> 3;
-      float2* sStats = reinterpret_cast<float2*>(sbias + GEMM_LN_STATS_OFF);      // [128] (mean, rstd)
-      const int M = p.rows_per_batch;
-      const int my_blocks = my_tiles / n_tiles;
-      auto block_row0 = [&](int mi) {
-        int mt, nt;
-        tile_coords(mi * n_tiles, mt, nt);
-        return mt * GEMM_BM;
-      };
-      auto ln_load = [&](float4 (&v)[LN384_V], int r0, int pass) {
-        const int row = r0 + ow * 32 + pass * 4 + grp;
-        const float4* xr = reinterpret_cast<const float4*>(p.ln_x + size_t(row < M ? row : 0) * 384);
-#pragma unroll
-        for (int i = 0; i < LN384_V; ++i) v[i] = row < M ? __ldg(xr + i * 8 + sub) : make_float4(0.f, 0.f, 0.f, 0.f);
-      };
-      int mi_phase = 0;
-      // k-block kb of the A block: columns kb*64 .. +63 of the warp's 32 rows = float4 numbers (2kb)*8 + sub and
-      // (2kb + 1)*8 + sub of each row, normalised with the stored statistics
-      auto ln_store_kb = [&](int r0, int kb) {
-        float4 v[8][2];
-#pragma unroll
-        for (int pass = 0; pass < 8; ++pass) {
-          const int row = r0 + ow * 32 + pass * 4 + grp;
-          const float4* xr = reinterpret_cast<const float4*>(p.ln_x + size_t(row < M ? row : 0) * 384) + kb * 16 + sub;
-          v[pass][0] = row < M ? __ldg(xr) : make_float4(0.f, 0.f, 0.f, 0.f);
-          v[pass][1] = row < M ? __ldg(xr + 8) : make_float4(0.f, 0.f, 0.f, 0.f);
-        }
-        mbar_wait(&a_empty[kb], (mi_phase & 1) ^ 1);   // the previous row block's last n-tile has read this k-block
-        uint8_t* blk = smem + size_t(kb) * GEMM_A_BYTES + (sub & 1) * 8;
-#pragma unroll
-        for (int pass = 0; pass < 8; ++pass) {
-          const int r = ow * 32 + pass * 4 + grp;    // row inside the block
-          const float2 st = sStats[r];
-          const bool live = r0 + r < M;
-#pragma unroll
-          for (int j = 0; j < 2; ++j) {
-            uint2 o = ln384_out_plain(v[pass][j], st.x, st.y);
-            if (!live) o = make_uint2(0u, 0u);
-            *reinterpret_cast<uint2*>(blk + r * 128 + ((((j * 8 + sub) >> 1) ^ (r & 7)) << 4)) = o;
-          }
-        }
-        fence_proxy_async_smem();                    // generic-proxy writes -> visible to the UMMA reads of the block
-        __syncwarp();
-        if (lane == 0) arrive_leader(&a_full[kb]);
-      };
-      for (int mi = 0; mi < my_blocks; ++mi) {
-        const int r0 = block_row0(mi);
-        float4 va[LN384_V], vb[LN384_V];
-        // (1) statistics: any time before the A block frees up (the previous row block is still being multiplied)
-        ln_load(va, r0, 0);
-#pragma unroll 1
-        for (int pass = 0; pass < 8; pass += 2) {
-          ln_load(vb, r0, pass + 1);
-          float mean, rstd;
-          ln384_stats(va, p.ln_eps, mean, rstd);
-          if (sub == 0) sStats[ow * 32 + pass * 4 + grp] = make_float2(mean, rstd);
-          if (pass + 2 < 8) ln_load(va, r0, pass + 2);
-          ln384_stats(vb, p.ln_eps, mean, rstd);
-          if (sub == 0) sStats[ow * 32 + (pass + 1) * 4 + grp] = make_float2(mean, rstd);
-        }
-        __syncwarp();                                // the statistics are read back by the lanes of this warp only
-        // (2) write, k-block by k-block as the last n-tile of the previous row block releases them (rows again: L2
-        // hits), so that the first MMAs of this row block start after a sixth of the block has been produced
-        mi_phase = mi;
-#pragma unroll 1
-        for (int kb = 0; kb < GEMM_RES_KB; ++kb) ln_store_kb(r0, kb);
-      }
     }
   } else {
     // ---------------- epilogue: thread <-> accumulator row ----------------

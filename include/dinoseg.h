@@ -192,11 +192,6 @@ int dinoseg_op_gemm(const void* A_bf16, const void* W_bf16, const float* bias, v
  * tiles, the W tile split between the two SMs) - how the qkv GEMM (and ViT-B's fc1 / fc2) of the forward are launched */
 int dinoseg_op_gemm_pair(const void* A, const void* W, const float* bias, void* out, int M, int N, int K, int ldo, int epi,
                          float col_scale, int scale_cols, void* stream);
-/* out[M, N] bf16 = (xhat W^T + bias) * (col < scale_cols ? col_scale : 1) with xhat = LayerNorm(x) WITHOUT its affine
- * transform (x fp32 [M, 384]; gamma / beta folded into W / bias by dinoseg_op_fold_ln): the CTA-pair GEMM that
- * normalises its own A operand - how norm1 -> qkv runs for ViT-S (reference vision_transformer.py:117, :133, :82) */
-int dinoseg_op_gemm_pair_ln(const float* x, const void* W_bf16, const float* bias, void* out_bf16, int M, int N, float eps,
-                            float col_scale, int scale_cols, void* stream);
 /* out[B*N, D] bf16 = softmax(q k^T) v over qkv[B, N, 3D] bf16; q carries dh^-0.5 * log2(e) already (the qkv GEMM's
  * epilogue applies it), i.e. the kernel computes P = 2^(q k^T) */
 int dinoseg_op_attention(const void* qkv_bf16, void* out_bf16, int B, int N, int H, void* stream);
@@ -235,9 +230,6 @@ int dinoseg_set_fused_mlp(dinoseg_t* h, int on);
 /* 1 (default where it applies: 'mlp' head, embed_dim 384): final LayerNorm -> layer_1 -> layer_2 -> layer_3 -> log_softmax
  * -> argmax -> p x p replication in ONE kernel (csrc/head.cuh); 0: the separate LayerNorm / GEMM / GEMM / tail kernels */
 int dinoseg_set_fused_head(dinoseg_t* h, int on);
-/* 1: LayerNorm1 of every block is computed by the qkv GEMM itself (CTA pairs, embed_dim 384 only) instead of its own kernel;
- * off by default (measured neutral, DESIGN.md section 4.2).  Same function, operands rounded to bf16 at the same points. */
-int dinoseg_set_fuse_ln1(dinoseg_t* h, int on);
 int dinoseg_op_layernorm(const float* x, const float* gamma, const float* beta, void* y_bf16, int M, int D,
                          float eps, void* stream);
 int dinoseg_op_posembed(const float* pos_src, float* out, int G0, int g, int D, void* stream);

@@ -480,35 +480,6 @@ def test_fused_head_matches_the_kernel_chain(variant, res, batch):
     assert torch.equal(low_only, low1) and torch.equal(lab_only, lab1)
 
 
-@pytest.mark.parametrize("variant", ["reference_init", "trained_like"])
-def test_layernorm1_inside_the_qkv_gemm_matches_the_two_kernel_path(variant):
-    """Opt-in form of norm1 -> qkv (reference vision_transformer.py:117, :133, :82): the CTA-pair GEMM normalises the fp32
-    tokens itself (gamma / beta folded into the qkv weight) instead of reading the LayerNorm kernel's bf16 output.  Same
-    function, but gamma is rounded into the bf16 weight instead of into the bf16 activations: the two paths differ from
-    each other by what each may differ from the fp32 reference (the tolerances of the golden-vector tests)."""
-    lib = _lib.load()
-    m, cfg, sd = _model("vit_small", 2, 21, variant)
-    x = synthetic.make_frames(3, 240, seed=11).cuda()
-    lp0, low0, _ = m.infer(x, want_logprobs=True, want_lowres=True)
-    n0 = m.last_launch_count()
-    assert lib.dinoseg_set_fuse_ln1(m._handle, 1) == 0
-    try:
-        lp1, low1, _ = m.infer(x, want_logprobs=True, want_lowres=True)
-        n1 = m.last_launch_count()
-    finally:
-        assert lib.dinoseg_set_fuse_ln1(m._handle, 0) == 0
-    torch.cuda.synchronize()
-    assert n1 == n0 - 2                                            # one LayerNorm launch less per block
-    rng = float(lp0.max() - lp0.min())
-    d = float((lp1 - lp0).abs().max())
-    _record(case=f"fuse_ln1_{variant}_240", max_abs_vs_two_kernels=d, range=rng)
-    if variant == "reference_init":
-        assert d <= TOL_ABS_REFINIT * max(1.0, rng), (d, rng)
-    else:
-        assert d <= TOL_REL_TRAINED * rng, (d, rng)
-    assert float((low1 == low0).float().mean()) >= 0.99
-
-
 def test_bench_dumps_the_label_maps_of_its_timed_path(tmp_path):
     """bench.py --dump-outputs: the float32 copy of the int64 label maps of the last timed step, equal to what
     DINOSeg.infer returns for the bench's seeded weights (seed 0) and frames (seed 1); --steps is the number of timed steps."""

@@ -224,41 +224,6 @@ def check_mlp_ln(name, M, pair=0):
                    update_absmax=scale, max_diff_fused_vs_two_kernels=(one - two).abs().max().item())
 
 
-def check_gemm_ln(name, M, N=1152):
-    """CTA-pair GEMM that normalises its own A operand (LayerNorm1 -> qkv: dinoseg_op_fold_ln + dinoseg_op_gemm_pair_ln)
-    against fp32 torch and against the two-kernel path (LayerNorm kernel, then the pair GEMM on its bf16 output)."""
-    torch, L, lib = _imports()
-    torch.manual_seed(9)
-    dev = "cuda"
-    x = torch.randn(M, 384, device=dev) * 1.5 + 0.2
-    x[min(3, M - 1)] *= 40.0                       # a row with a large mean / spread
-    g = 1.0 + 0.1 * torch.randn(384, device=dev)
-    b = 0.1 * torch.randn(384, device=dev)
-    W = torch.randn(N, 384, device=dev) * 0.05
-    bias = 0.1 * torch.randn(N, device=dev)
-    scale_cols = 384 if N >= 384 else 0
-    F = torch.nn.functional
-    ref = F.linear(F.layer_norm(x, (384,), g, b, 1e-6), W, bias)                  # fp32 throughout
-    ref[:, :scale_cols] *= 0.125
-    A = torch.zeros(M, 384, device=dev, dtype=torch.bfloat16)
-    rc0 = lib.dinoseg_op_layernorm(_ptr(x), _ptr(g), _ptr(b), _ptr(A), M, 384, 1e-6, None)
-    two = torch.zeros(M, N, device=dev, dtype=torch.bfloat16)
-    Wb = W.to(torch.bfloat16)
-    rc1 = lib.dinoseg_op_gemm_pair(_ptr(A), _ptr(Wb), _ptr(bias), _ptr(two), M, N, 384, N, 0, 0.125, scale_cols, None)
-    Wf = torch.zeros(N, 384, device=dev, dtype=torch.bfloat16)
-    bf = torch.zeros(N, device=dev)
-    rc2 = lib.dinoseg_op_fold_ln(_ptr(W), _ptr(bias), _ptr(g), _ptr(b), N, 384, _ptr(Wf), _ptr(bf), None)
-    one = torch.full((M, N), float("nan"), device=dev, dtype=torch.bfloat16)
-    rc3 = lib.dinoseg_op_gemm_pair_ln(_ptr(x), _ptr(Wf), _ptr(bf), _ptr(one), M, N, 1e-6, 0.125, scale_cols, None)
-    torch.cuda.synchronize()
-    scale = ref.abs().max().item()
-    err1, err2 = (one.float() - ref).abs().max().item(), (two.float() - ref).abs().max().item()
-    ok = rc0 == 0 and rc1 == 0 and rc2 == 0 and rc3 == 0 and err1 <= 1e-2 * scale and err2 <= 1e-2 * scale \
-        and bool(torch.isfinite(one.float()).all())
-    return _report(name, ok, rc=[rc0, rc1, rc2, rc3], max_abs_err_fused=err1, max_abs_err_two_kernels=err2, ref_absmax=scale,
-                   max_diff_fused_vs_two_kernels=(one.float() - two.float()).abs().max().item())
-
-
 def check_layernorm(name, M, D):
     torch, L, lib = _imports()
     torch.manual_seed(3)
@@ -380,10 +345,6 @@ def _checks():
         "mlp_ln_multi": lambda: check_mlp_ln("mlp_ln_multi", 148 * 128 * 2 + 77),
         "mlp_ln_pair_ragged": lambda: check_mlp_ln("mlp_ln_pair_ragged", 901, 1),
         "mlp_ln_pair_multi": lambda: check_mlp_ln("mlp_ln_pair_multi", 148 * 128 * 3 + 300, 1),
-        "gemm_ln_small": lambda: check_gemm_ln("gemm_ln_small", 77),
-        "gemm_ln_ragged": lambda: check_gemm_ln("gemm_ln_ragged", 901),
-        "gemm_ln_odd_blocks": lambda: check_gemm_ln("gemm_ln_odd_blocks", 128 * 5 + 1),
-        "gemm_ln_multi": lambda: check_gemm_ln("gemm_ln_multi", 148 * 128 * 3 + 300),
     }
 
 
@@ -394,7 +355,6 @@ def check_names():
         "gemm_resid_k1536", "gemm_patch", "gemm_head", "gemm_big", "attn_1tile", "attn_ragged_small", "attn_2tiles",
         "attn_901", "attn_3601", "attn_vitb_901", "mlp_1block", "mlp_ragged", "mlp_multi", "mlp_pair_1block", "mlp_pair_ragged", "mlp_pair_multi",
         "mlp_ln_ragged", "mlp_ln_multi", "mlp_ln_pair_ragged", "mlp_ln_pair_multi",
-        "gemm_ln_small", "gemm_ln_ragged", "gemm_ln_odd_blocks", "gemm_ln_multi",
     ]
 
 
