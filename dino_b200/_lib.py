@@ -45,6 +45,10 @@ SIGNATURES = {
     "dinoseg_predict_host_wait": (C.c_int, [C.c_void_p, C.c_int64]),
     "dinoseg_set_host_chunk": (C.c_int, [C.c_void_p, C.c_int]),
     "dinoseg_cls_attention": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "dinoseg_features": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_size_t,
+                                   C.c_void_p]),
+    "dinoseg_features_u8": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float),
+                                      C.POINTER(C.c_float), C.c_int, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
     "dinoseg_argmax_replicate": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p,
                                            C.c_void_p, C.c_void_p]),
     "dinoseg_copy_buffer": (C.c_int64, [C.c_void_p, C.c_char_p, C.c_void_p, C.c_size_t, C.c_void_p]),
@@ -85,6 +89,8 @@ SIGNATURES = {
     "dinoseg_set_fused_head": (C.c_int, [C.c_void_p, C.c_int]),
     "dinoseg_op_layernorm": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
                                        C.c_float, C.c_void_p]),
+    "dinoseg_op_layernorm_f32": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int,
+                                           C.c_float, C.c_void_p]),
     "dinoseg_op_posembed": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p]),
     "dinoseg_op_im2col": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     "dinoseg_op_f32_to_bf16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),

@@ -331,10 +331,20 @@ cudaError_t launch_layernorm(const float* x, const float* g, const float* b, __n
                              bool split, cudaStream_t s) {
   const int rows_per_block = 8;
   dim3 grid((M + rows_per_block - 1) / rows_per_block);
-  if (D == 384 && !split) layernorm384_bf16_kernel<<<(M + 31) / 32, 256, 0, s>>>(x, g, b, y, M, eps);
-  else if (D == 768 && !split) layernorm_bf16_kernel<768, false><<<grid, 256, 0, s>>>(x, g, b, y, M, eps);
-  else if (D == 384 && split) layernorm_bf16_kernel<384, true><<<grid, 256, 0, s>>>(x, g, b, y, M, eps);
-  else if (D == 768 && split) layernorm_bf16_kernel<768, true><<<grid, 256, 0, s>>>(x, g, b, y, M, eps);
+  if (D == 384 && !split) layernorm384_kernel<__nv_bfloat16><<<(M + 31) / 32, 256, 0, s>>>(x, g, b, y, M, eps);
+  else if (D == 768 && !split) layernorm_kernel<768, false, __nv_bfloat16><<<grid, 256, 0, s>>>(x, g, b, y, M, eps);
+  else if (D == 384 && split) layernorm_kernel<384, true, __nv_bfloat16><<<grid, 256, 0, s>>>(x, g, b, y, M, eps);
+  else if (D == 768 && split) layernorm_kernel<768, true, __nv_bfloat16><<<grid, 256, 0, s>>>(x, g, b, y, M, eps);
+  else return cudaErrorInvalidValue;
+  return cudaGetLastError();
+}
+
+// fp32 output (backbone features: dino.norm applied to the residual stream), same kernels as above
+cudaError_t launch_layernorm_f32(const float* x, const float* g, const float* b, float* y, int M, int D, float eps,
+                                 cudaStream_t s) {
+  if (M <= 0) return cudaErrorInvalidValue;
+  if (D == 384) layernorm384_kernel<float><<<(M + 31) / 32, 256, 0, s>>>(x, g, b, y, M, eps);
+  else if (D == 768) layernorm_kernel<768, false, float><<<(M + 7) / 8, 256, 0, s>>>(x, g, b, y, M, eps);
   else return cudaErrorInvalidValue;
   return cudaGetLastError();
 }
@@ -1101,11 +1111,20 @@ cudaError_t launch_head_fused(dinoseg_t* h, const float* x, int M, float* logpro
   return cudaGetLastError();
 }
 
+// Backbone features requested from forward_impl: after every block i >= first, the final LayerNorm (dino.norm) of the
+// residual stream goes to out[i - first] (fp32 [M, D] slices); backbone_only ends the pass before the head.
+struct FeatureReq {
+  float* out = nullptr;
+  int first = 0;
+  bool backbone_only = false;
+};
+
 // Launch sequence of one forward pass over `batch` frames on the buffers of `w` (already bound).
 // `frames` are normalised fp32 NCHW frames, or (frames == nullptr) `frames_u8` raw uint8 HWC frames that are resized
-// and normalised on the fly (pp).
+// and normalised on the fly (pp).  `feat` (optional): backbone features to emit on the way.
 static int forward_impl(dinoseg_t* h, WorkBufs& w, const float* frames, const uint8_t* frames_u8, const PreprocParams* pp,
-                        int batch, float* logprobs, uint8_t* lowres, int64_t* labels, cudaStream_t s) {
+                        int batch, float* logprobs, uint8_t* lowres, int64_t* labels, cudaStream_t s,
+                        const FeatureReq* feat = nullptr) {
   if (h->res == 0) DSG_FAIL(h, "dinoseg_forward: call dinoseg_set_resolution first");
   if (dinoseg_missing_weights(h) != 0) {
     std::string miss;
@@ -1237,8 +1256,15 @@ static int forward_impl(dinoseg_t* h, WorkBufs& w, const float* frames, const ui
         ++n;
       }
     }
+    if (feat && i >= feat->first) {
+      // before anything else touches x (the kernel-chain head reuses its buffer for relu(layer_2))
+      LaunchScope ls(h, K_LN, s);
+      DSG_CUDA(h, launch_layernorm_f32(w.x, h->norm_g, h->norm_b, feat->out + size_t(i - feat->first) * M * D, M, D, eps, s));
+      ++n;
+    }
     if (stop == 4 + 3 * i) { h->launches = n; return 0; }
   }
+  if (feat && feat->backbone_only) { h->launches = n; return 0; }
 
   // ---- final norm + head (vision_transformer.py:243, pl_torch_modules.py:243-255) ----
   // The head runs in "bf16x3" precision (operands split into hi + lo bf16 parts, three-fold K): its plain
@@ -1823,6 +1849,44 @@ int dinoseg_cls_attention(dinoseg_t* h, const float* frames, int batch, float* a
   return 0;
 }
 
+// Backbone features of the last min(n_last, n_blocks) blocks in ONE pass over the blocks (no head).
+static int features_impl(dinoseg_t* h, const float* frames, const uint8_t* frames_u8, const PreprocParams* pp, int batch,
+                         int n_last, float* out, void* workspace, size_t workspace_bytes, void* stream, const char* what) {
+  if (h->res == 0) DSG_FAIL(h, "%s: call dinoseg_set_resolution first", what);
+  if ((!frames && !frames_u8) || batch <= 0 || !workspace) DSG_FAIL(h, "%s: bad arguments", what);
+  if (!out) DSG_FAIL(h, "%s: out is NULL", what);
+  if (n_last < 1) DSG_FAIL(h, "%s: n_last must be >= 1 (got %d)", what, n_last);
+  if (h->cfg.n_blocks < 1) DSG_FAIL(h, "%s: the model has no transformer block", what);
+  DSG_CUDA(h, cudaSetDevice(h->device));
+  if (bind_workspace(h, h->user, workspace, workspace_bytes, batch) != 0) return -1;
+  FeatureReq req;
+  req.out = out;
+  req.first = h->cfg.n_blocks - std::min(n_last, h->cfg.n_blocks);
+  req.backbone_only = true;
+  const int saved = h->debug_stop;   // a debug stop would leave slices of `out` unwritten
+  h->debug_stop = 0;
+  const int rc = forward_impl(h, h->user, frames, frames_u8, pp, batch, nullptr, nullptr, nullptr,
+                              static_cast<cudaStream_t>(stream), &req);
+  h->debug_stop = saved;
+  return rc;
+}
+
+int dinoseg_features(dinoseg_t* h, const float* frames, int batch, int n_last, float* out, void* workspace,
+                     size_t workspace_bytes, void* stream) {
+  if (!h) return -1;
+  return features_impl(h, frames, nullptr, nullptr, batch, n_last, out, workspace, workspace_bytes, stream,
+                       "dinoseg_features");
+}
+
+int dinoseg_features_u8(dinoseg_t* h, const uint8_t* frames, int batch, int src_h, int src_w, const float* mean,
+                        const float* std_, int n_last, float* out, void* workspace, size_t workspace_bytes, void* stream) {
+  if (!h) return -1;
+  PreprocParams pp;
+  if (make_preproc(h, src_h, src_w, mean, std_, &pp) != 0) return -1;
+  return features_impl(h, nullptr, frames, &pp, batch, n_last, out, workspace, workspace_bytes, stream,
+                       "dinoseg_features_u8");
+}
+
 int dinoseg_set_fused_mlp(dinoseg_t* h, int on) {
   if (!h) return -1;
   if (on && !(h->cfg.embed_dim == MLP_D && h->cfg.mlp_hidden == MLP_HID))
@@ -1916,6 +1980,12 @@ int dinoseg_op_layernorm(const float* x, const float* gamma, const float* beta, 
                          void* stream) {
   return launch_layernorm(x, gamma, beta, static_cast<__nv_bfloat16*>(y), M, D, eps, false,
                           static_cast<cudaStream_t>(stream)) == cudaSuccess ? 0 : -1;
+}
+
+int dinoseg_op_layernorm_f32(const float* x, const float* gamma, const float* beta, float* y, int M, int D, float eps,
+                             void* stream) {
+  if (!x || !gamma || !beta || !y) return -1;
+  return launch_layernorm_f32(x, gamma, beta, y, M, D, eps, static_cast<cudaStream_t>(stream)) == cudaSuccess ? 0 : -1;
 }
 
 int dinoseg_op_posembed(const float* pos_src, float* out, int G0, int g, int D, void* stream) {

@@ -1,6 +1,8 @@
 // Memory-bound kernels of the DINOSeg hot path (HBM-bound: coalesced 16-byte accesses,
 // warp-shuffle reductions, no tensor cores).
 #pragma once
+#include <type_traits>
+
 #include "ptx.cuh"
 
 namespace dsg {
@@ -246,14 +248,21 @@ __device__ __forceinline__ void ln384_stats(const float4 (&v)[LN384_V], float ep
   sq += __shfl_xor_sync(0xffffffffu, sq, 4);
   rstd = rsqrtf(sq * (1.0f / 384.0f) + eps);
 }
-// normalised, affine-transformed float4 number i*8 + sub of the row -> four bf16 (two packed words)
-__device__ __forceinline__ uint2 ln384_out(const float4& v, float mean, float rstd, const float4& gm, const float4& bt) {
+// normalised, affine-transformed float4 number i of the row -> four outputs at float4 position i of the output row:
+// bf16 (two packed words, one 8-byte store) or fp32 (one 16-byte store)
+__device__ __forceinline__ void ln_out4(__nv_bfloat16* yr, int i, const float4& v, float mean, float rstd,
+                                        const float4& gm, const float4& bt) {
   const float a = (v.x - mean) * rstd * gm.x + bt.x, b = (v.y - mean) * rstd * gm.y + bt.y;
   const float c = (v.z - mean) * rstd * gm.z + bt.z, d = (v.w - mean) * rstd * gm.w + bt.w;
   uint2 o;
   o.x = pack_bf16x2(a, b);
   o.y = pack_bf16x2(c, d);
-  return o;
+  reinterpret_cast<uint2*>(yr)[i] = o;
+}
+__device__ __forceinline__ void ln_out4(float* yr, int i, const float4& v, float mean, float rstd, const float4& gm,
+                                        const float4& bt) {
+  reinterpret_cast<float4*>(yr)[i] = make_float4((v.x - mean) * rstd * gm.x + bt.x, (v.y - mean) * rstd * gm.y + bt.y,
+                                                 (v.z - mean) * rstd * gm.z + bt.z, (v.w - mean) * rstd * gm.w + bt.w);
 }
 
 // normalised float4 WITHOUT the affine transform (the consumer's weights carry gamma and beta: fold_ln_weight_kernel)
@@ -306,10 +315,12 @@ fold_split_ln_weight_kernel(const float* __restrict__ W, const float* __restrict
   if (lane == 0) bf[warp] = b[warp] + acc;
 }
 
-// D = 384, plain bf16 output: four rows per warp (eight lanes per row), 32 rows per 256-thread block
+// D = 384, plain output (OutT = bf16: GEMM operand; fp32: backbone features): four rows per warp (eight lanes per row),
+// 32 rows per 256-thread block
+template <typename OutT>
 __global__ void __launch_bounds__(256)
-layernorm384_bf16_kernel(const float* __restrict__ x, const float* __restrict__ gamma, const float* __restrict__ beta,
-                         __nv_bfloat16* __restrict__ y, int M, float eps) {
+layernorm384_kernel(const float* __restrict__ x, const float* __restrict__ gamma, const float* __restrict__ beta,
+                    OutT* __restrict__ y, int M, float eps) {
   const int sub = threadIdx.x & 7;
   const int row = blockIdx.x * 32 + (threadIdx.x >> 3);
   const bool live = row < M;
@@ -320,19 +331,21 @@ layernorm384_bf16_kernel(const float* __restrict__ x, const float* __restrict__ 
   float mean, rstd;
   ln384_stats(v, eps, mean, rstd);
   if (!live) return;
-  uint2* yr = reinterpret_cast<uint2*>(y + size_t(row) * 384);
+  OutT* yr = y + size_t(row) * 384;
 #pragma unroll
   for (int i = 0; i < LN384_V; ++i)
-    yr[i * 8 + sub] = ln384_out(v[i], mean, rstd, __ldg(reinterpret_cast<const float4*>(gamma) + i * 8 + sub),
-                                __ldg(reinterpret_cast<const float4*>(beta) + i * 8 + sub));
+    ln_out4(yr, i * 8 + sub, v[i], mean, rstd, __ldg(reinterpret_cast<const float4*>(gamma) + i * 8 + sub),
+            __ldg(reinterpret_cast<const float4*>(beta) + i * 8 + sub));
 }
 
-// SPLIT: y is [M, 2*D] = [hi | lo] (bf16x3 operand of the head GEMM, see split_weight_kernel).
-template <int D, bool SPLIT>
+// One warp per row.  SPLIT (bf16 only): y is [M, 2*D] = [hi | lo] (bf16x3 operand of the head GEMM, see
+// split_weight_kernel).
+template <int D, bool SPLIT, typename OutT>
 __global__ void __launch_bounds__(256)
-layernorm_bf16_kernel(const float* __restrict__ x, const float* __restrict__ gamma, const float* __restrict__ beta,
-                      __nv_bfloat16* __restrict__ y, int M, float eps) {
+layernorm_kernel(const float* __restrict__ x, const float* __restrict__ gamma, const float* __restrict__ beta,
+                 OutT* __restrict__ y, int M, float eps) {
   static_assert(D % 128 == 0, "D must be a multiple of 128");
+  static_assert(!SPLIT || std::is_same<OutT, __nv_bfloat16>::value, "the split output is bf16");
   constexpr int V = D / 128;
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int row = blockIdx.x * (blockDim.x >> 5) + warp;
@@ -357,22 +370,25 @@ layernorm_bf16_kernel(const float* __restrict__ x, const float* __restrict__ gam
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) sq += __shfl_xor_sync(0xffffffffu, sq, o);
   const float rstd = rsqrtf(sq * (1.0f / D) + eps);
-  uint2* yr = reinterpret_cast<uint2*>(y + size_t(row) * (SPLIT ? 2 * D : D));
+  OutT* yr = y + size_t(row) * (SPLIT ? 2 * D : D);
 #pragma unroll
   for (int i = 0; i < V; ++i) {
     const float4 gm = __ldg(reinterpret_cast<const float4*>(gamma) + i * 32 + lane);
     const float4 bt = __ldg(reinterpret_cast<const float4*>(beta) + i * 32 + lane);
-    const float a = (v[i].x - mean) * rstd * gm.x + bt.x, b = (v[i].y - mean) * rstd * gm.y + bt.y;
-    const float c = (v[i].z - mean) * rstd * gm.z + bt.z, d = (v[i].w - mean) * rstd * gm.w + bt.w;
-    uint2 o;
-    o.x = pack_bf16x2(a, b);
-    o.y = pack_bf16x2(c, d);
-    yr[i * 32 + lane] = o;
     if constexpr (SPLIT) {
+      const float a = (v[i].x - mean) * rstd * gm.x + bt.x, b = (v[i].y - mean) * rstd * gm.y + bt.y;
+      const float c = (v[i].z - mean) * rstd * gm.z + bt.z, d = (v[i].w - mean) * rstd * gm.w + bt.w;
+      uint2 o;
+      o.x = pack_bf16x2(a, b);
+      o.y = pack_bf16x2(c, d);
+      uint2* yw = reinterpret_cast<uint2*>(yr);
+      yw[i * 32 + lane] = o;
       uint2 l;
       l.x = pack_bf16x2(a - __uint_as_float(o.x << 16), b - __uint_as_float(o.x & 0xffff0000u));
       l.y = pack_bf16x2(c - __uint_as_float(o.y << 16), d - __uint_as_float(o.y & 0xffff0000u));
-      yr[D / 4 + i * 32 + lane] = l;
+      yw[D / 4 + i * 32 + lane] = l;
+    } else {
+      ln_out4(yr, i * 32 + lane, v[i], mean, rstd, gm, bt);
     }
   }
 }

@@ -10,6 +10,7 @@ from __future__ import annotations
 
 import ctypes as C
 import io
+import numbers
 import pickle
 import types
 import warnings
@@ -26,8 +27,8 @@ from .transforms import IMAGENET_MEAN, IMAGENET_STD, get_transforms
 
 # ------------------------------------------------------------------------------------------
 # Parameter containers with the reference's state_dict names (vision_transformer.py:163-191).
-# They are never called: they only hold tensors (and give PyTorch's default initialisers, which
-# is what the reference relies on for the conv and the head).
+# They compute nothing themselves: they hold tensors (and give PyTorch's default initialisers, which
+# is what the reference relies on for the conv and the head); _Backbone's forward goes to the library.
 # ------------------------------------------------------------------------------------------
 class _Attention(nn.Module):
     def __init__(self, dim):
@@ -78,14 +79,29 @@ class _Backbone(nn.Module):
         nn.init.trunc_normal_(self.cls_token, std=.02)
         self.apply(self._init_weights)
 
+    def _model(self):
+        owner = self._owner() if self._owner is not None else None
+        if owner is None:
+            raise RuntimeError("backbone is not attached to a DINOSeg model")
+        return owner
+
+    def forward(self, x):
+        """VisionTransformer.forward (vision_transformer.py:237-248) for all tokens: fp32 [B,3,r,r] (normalised, on the
+        model's device) -> fp32 [B, N, D], N = (r/8)^2 + 1, CLS token first, after the final norm.  Runs on the GPU
+        through DINOSeg.features; the head does not run."""
+        return self._model().features(x, 1)[0]
+
+    def get_intermediate_layers(self, x, n=1):
+        """vision_transformer.py:282-290: list of min(n, n_blocks) fp32 [B, N, D] tensors, oldest block first, each the
+        final norm of the residual stream after one of the last n blocks (one pass over the blocks).  The last element
+        equals forward(x) bit for bit."""
+        return list(self._model().features(x, n).unbind(0))
+
     def get_last_selfattention(self, x):
         """Reference vision_transformer.py:273-280 returns the last block's attention [B, H, N, N]; its only caller
         (visualize_attention.py:46-54) reads the CLS row `[0, :, 0, 1:]`.  Here only that row is materialised:
         the result has shape [B, H, 1, N] (the full matrix is 311 MB per frame at 480 px and is never formed)."""
-        owner = self._owner() if self._owner is not None else None
-        if owner is None:
-            raise RuntimeError("backbone is not attached to a DINOSeg model")
-        return owner.cls_attention(x).unsqueeze(2)
+        return self._model().cls_attention(x).unsqueeze(2)
 
     @staticmethod
     def _init_weights(m):
@@ -398,6 +414,49 @@ class DINOSeg(nn.Module):
         rc = lib.dinoseg_cls_attention(self._handle, x.data_ptr(), b, out.data_ptr(), ws.data_ptr(), ws.numel(),
                                        self._stream())
         self._check(rc, "dinoseg_cls_attention")
+        return out
+
+    @torch.no_grad()
+    def features(self, x, n=1, resolution=None):
+        """Backbone features of the last n blocks in one pass (no head): a device fp32 tensor [min(n, n_blocks), B, N, D],
+        N = (r/8)^2 + 1 with the CLS token first; slice k is the final norm (dino.norm) of the residual stream after
+        block n_blocks - min(n, n_blocks) + k (vision_transformer.py:282-290).  x: device fp32 [B,3,r,r] (normalised),
+        or device uint8 [B,H,W,3] raw RGB frames resized to `resolution` (default self.resolution) and normalised as
+        in infer_u8.  Asynchronous on the current stream."""
+        if not isinstance(n, numbers.Integral) or n < 1:
+            raise ValueError(f"n must be a positive integer, got {n!r}")
+        n = int(n)
+        lib = self._ensure_handle()
+        if x.device != self.device:
+            raise ValueError(f"frames are on {x.device}, model on {self.device}")
+        raw = x.dtype == torch.uint8
+        if raw:
+            if x.dim() != 4 or x.shape[3] != 3:
+                raise ValueError(f"expected uint8 frames of shape [B,H,W,3], got {tuple(x.shape)}")
+            res = int(self.resolution if resolution is None else resolution)
+        else:
+            if x.dim() != 4 or x.shape[1] != 3 or x.shape[2] != x.shape[3]:
+                raise ValueError(f"expected frames of shape [B,3,r,r], got {tuple(x.shape)}")
+            res = int(x.shape[2])
+            if resolution is not None and int(resolution) != res:
+                raise ValueError(f"resolution {resolution} given for frames of size {res}")
+            x = x.float()
+        x = x.contiguous()
+        b = int(x.shape[0])
+        self._ensure_resolution(lib, res)
+        ws = self._ensure_workspace(lib, b)
+        n_out = min(n, self.n_blocks)
+        out = torch.empty((n_out, b, (res // 8) ** 2 + 1, self.mlp_input_dim), dtype=torch.float32, device=self.device)
+        if raw:
+            mean = (C.c_float * 3)(*IMAGENET_MEAN)
+            std = (C.c_float * 3)(*IMAGENET_STD)
+            rc = lib.dinoseg_features_u8(self._handle, x.data_ptr(), b, int(x.shape[1]), int(x.shape[2]), mean, std, n,
+                                         out.data_ptr(), ws.data_ptr(), ws.numel(), self._stream())
+            self._check(rc, "dinoseg_features_u8")
+        else:
+            rc = lib.dinoseg_features(self._handle, x.data_ptr(), b, n, out.data_ptr(), ws.data_ptr(), ws.numel(),
+                                      self._stream())
+            self._check(rc, "dinoseg_features")
         return out
 
     def forward(self, x):

@@ -138,6 +138,19 @@ int dinoseg_get_pair_kernels(const dinoseg_t* h);   /* bit 0: GEMMs, bit 1: fuse
 int dinoseg_cls_attention(dinoseg_t* h, const float* frames, int batch, float* attn, void* workspace,
                           size_t workspace_bytes, void* stream);
 
+/* Backbone features: VisionTransformer.get_intermediate_layers(x, n_last) (vision_transformer.py:282-290) in one pass
+ * over the blocks, without the head.  out: device fp32 [min(n_last, n_blocks), batch, N, D], N = (r/8)^2 + 1 (CLS
+ * token first); slice k = dino.norm (eps ln_eps) applied to the residual stream after block
+ * n_blocks - min(n_last, n_blocks) + k, so the last slice is what VisionTransformer.forward returns for all tokens.
+ * frames: device fp32 [batch,3,r,r] (normalised).  Workspace as for dinoseg_forward (dinoseg_workspace_bytes).
+ * n_last < 1, out == NULL, no resolution set, a model without blocks or a too small workspace: error. */
+int dinoseg_features(dinoseg_t* h, const float* frames, int batch, int n_last, float* out, void* workspace,
+                     size_t workspace_bytes, void* stream);
+/* The same on raw uint8 HWC frames [batch, src_h, src_w, 3], resized and normalised as in dinoseg_forward_u8. */
+int dinoseg_features_u8(dinoseg_t* h, const uint8_t* frames_u8, int batch, int src_h, int src_w, const float* mean,
+                        const float* std_, int n_last, float* out, void* workspace, size_t workspace_bytes,
+                        void* stream);
+
 /* Controller-side reduction on the label map (the step after predict() in the robot pipeline, reference
  * docs/index.html "Controller": left / right obstacle masks for the potential-field controller).
  * lowres: device uint8 [batch, g, g] as written by dinoseg_forward; the output map is (g*p) x (g*p).
@@ -232,6 +245,9 @@ int dinoseg_set_fused_mlp(dinoseg_t* h, int on);
 int dinoseg_set_fused_head(dinoseg_t* h, int on);
 int dinoseg_op_layernorm(const float* x, const float* gamma, const float* beta, void* y_bf16, int M, int D,
                          float eps, void* stream);
+/* y[M,D] fp32 = LayerNorm(x) * gamma + beta, D = 384 or 768: the kernel behind dinoseg_features */
+int dinoseg_op_layernorm_f32(const float* x, const float* gamma, const float* beta, float* y, int M, int D,
+                             float eps, void* stream);
 int dinoseg_op_posembed(const float* pos_src, float* out, int G0, int g, int D, void* stream);
 int dinoseg_op_im2col(const float* frames, void* A_bf16, int B, int g, void* stream);
 int dinoseg_op_f32_to_bf16(const float* in, void* out_bf16, size_t n, void* stream);
