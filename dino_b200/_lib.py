@@ -30,6 +30,7 @@ SIGNATURES = {
     "dinoseg_set_weight": (C.c_int, [C.c_void_p, C.c_char_p, C.c_void_p, C.POINTER(C.c_int64), C.c_int, C.c_void_p]),
     "dinoseg_missing_weights": (C.c_int, [C.c_void_p]),
     "dinoseg_set_resolution": (C.c_int, [C.c_void_p, C.c_int, C.c_void_p]),
+    "dinoseg_set_resolution_hw": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_void_p]),
     "dinoseg_workspace_bytes": (C.c_size_t, [C.c_void_p, C.c_int]),
     "dinoseg_forward": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
                                   C.c_void_p, C.c_size_t, C.c_void_p]),

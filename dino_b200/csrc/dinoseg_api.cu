@@ -349,27 +349,32 @@ cudaError_t launch_layernorm_f32(const float* x, const float* g, const float* b,
   return cudaGetLastError();
 }
 
-cudaError_t launch_posembed(const float* pos_src, float* out, int G0, int g, int D, cudaStream_t s) {
-  if (g == G0) {
-    // reference vision_transformer.py:205-206: same grid -> table returned unchanged
+// gh x gw patch grid (gh rows, gw columns)
+cudaError_t launch_posembed(const float* pos_src, float* out, int G0, int gh, int gw, int D, cudaStream_t s) {
+  if (gh == G0 && gw == G0) {
+    // reference vision_transformer.py:205-206 (npatch == N and w == h): same grid -> table returned unchanged.  A
+    // rectangle with gh*gw == G0*G0 (14 x 56) is resampled.
     return cudaMemcpyAsync(out, pos_src, size_t(G0 * G0 + 1) * D * sizeof(float), cudaMemcpyDeviceToDevice, s);
   }
-  const double sf = (double(g) + 0.1) / double(G0);  // reference :214-217 (python double)
-  const float rscale = float(1.0 / sf);              // ATen compute_scales_value<float>
-  const size_t total = size_t(g * g + 1) * D;
-  posembed_bicubic_kernel<<<unsigned((total + 255) / 256), 256, 0, s>>>(pos_src, out, G0, g, D, rscale);
+  // reference :212-217 (python doubles): scale_factor = ((gh + 0.1) / G0, (gw + 0.1) / G0), the first for the rows
+  // (its `w` is x.shape[2]); ATen compute_scales_value<float> per axis
+  const float rscale_y = float(1.0 / ((double(gh) + 0.1) / double(G0)));
+  const float rscale_x = float(1.0 / ((double(gw) + 0.1) / double(G0)));
+  const size_t total = size_t(gh * gw + 1) * D;
+  posembed_bicubic_kernel<<<unsigned((total + 255) / 256), 256, 0, s>>>(pos_src, out, G0, gh, gw, D, rscale_y, rscale_x);
   return cudaGetLastError();
 }
 
-cudaError_t launch_im2col(const float* frames, __nv_bfloat16* A, int B, int g, cudaStream_t s) {
-  const size_t total = size_t(B) * 3 * g * 4 * g;
-  im2col_patch8_kernel<<<unsigned((total + 255) / 256), 256, 0, s>>>(frames, A, B, g);
+cudaError_t launch_im2col(const float* frames, __nv_bfloat16* A, int B, int gh, int gw, cudaStream_t s) {
+  const size_t total = size_t(B) * 3 * gh * 4 * gw;
+  im2col_patch8_kernel<<<unsigned((total + 255) / 256), 256, 0, s>>>(frames, A, B, gh, gw);
   return cudaGetLastError();
 }
 
-cudaError_t launch_im2col_u8(const uint8_t* frames, __nv_bfloat16* A, int B, int g, const PreprocParams& pp, cudaStream_t s) {
-  const size_t total = size_t(B) * 3 * (g * 8) * g;
-  im2col_u8_kernel<<<unsigned((total + 255) / 256), 256, 0, s>>>(frames, A, B, g, pp);
+cudaError_t launch_im2col_u8(const uint8_t* frames, __nv_bfloat16* A, int B, int gh, int gw, const PreprocParams& pp,
+                             cudaStream_t s) {
+  const size_t total = size_t(B) * 3 * (gh * 8) * gw;
+  im2col_u8_kernel<<<unsigned((total + 255) / 256), 256, 0, s>>>(frames, A, B, gh, gw, pp);
   return cudaGetLastError();
 }
 
@@ -404,10 +409,10 @@ struct WeightSlot {
 };
 
 // One activation workspace carved into the buffers of a forward pass, with the tensor maps that
-// describe them (valid for one (base pointer, batch, resolution) binding).
+// describe them (valid for one (base pointer, batch, height, width) binding).
 struct WorkBufs {
   void* base = nullptr;
-  int batch = 0, res = 0;
+  int batch = 0, res_h = 0, res_w = 0;
   float* x = nullptr;               // fp32 residual stream [B*N, D]
   __nv_bfloat16* abuf = nullptr;    // bf16 GEMM A operand [B*N, D] (LayerNorm / attention output)
   __nv_bfloat16* qkv = nullptr;     // bf16 [B*N, 3D]
@@ -546,8 +551,9 @@ struct dinoseg {
   std::set<std::string> have;
   std::vector<void*> allocs;
 
-  // resolution state
-  int res = 0, g = 0, P = 0, Ntok = 0, p_rep = 0;
+  // resolution state: res_h x res_w pixels, gh x gw patches (0 = not set).  Label maps (p_rep > 0) exist for square
+  // grids only.
+  int res_h = 0, res_w = 0, gh = 0, gw = 0, P = 0, Ntok = 0, p_rep = 0;
   float* pos = nullptr;
   size_t pos_cap = 0;
 
@@ -653,7 +659,7 @@ int bind_workspace(dinoseg* h, WorkBufs& w, void* ws, size_t ws_bytes, int batch
   const WsLayout L = ws_layout(h, batch);
   if (ws_bytes < L.total) DSG_FAIL(h, "workspace too small: %zu < %zu bytes", ws_bytes, L.total);
   if ((reinterpret_cast<uintptr_t>(ws) & 1023) != 0) DSG_FAIL(h, "workspace must be 1024-byte aligned");
-  if (w.base == ws && w.batch == batch && w.res == h->res) return 0;
+  if (w.base == ws && w.batch == batch && w.res_h == h->res_h && w.res_w == h->res_w) return 0;
   uint8_t* base = static_cast<uint8_t*>(ws);
   w.x = reinterpret_cast<float*>(base + L.x);
   w.abuf = reinterpret_cast<__nv_bfloat16*>(base + L.abuf);
@@ -684,7 +690,8 @@ int bind_workspace(dinoseg* h, WorkBufs& w, void* ws, size_t ws_bytes, int batch
   if (!ok) DSG_FAIL(h, "cuTensorMapEncodeTiled failed for the workspace tensor maps");
   w.base = ws;
   w.batch = batch;
-  w.res = h->res;
+  w.res_h = h->res_h;
+  w.res_w = h->res_w;
   return 0;
 }
 
@@ -932,13 +939,17 @@ int dinoseg_missing_weights(const dinoseg_t* h) {
 }
 
 int dinoseg_set_resolution(dinoseg_t* h, int resolution, void* stream) {
+  return dinoseg_set_resolution_hw(h, resolution, resolution, stream);
+}
+
+int dinoseg_set_resolution_hw(dinoseg_t* h, int height, int width, void* stream) {
   if (!h) return -1;
-  if (resolution <= 0 || resolution % 8 != 0) DSG_FAIL(h, "Resolution should be a multiple of 8.");
+  if (height <= 0 || width <= 0 || height % 8 != 0 || width % 8 != 0) DSG_FAIL(h, "Resolution should be a multiple of 8.");
   if (!h->have.count("dino.pos_embed")) DSG_FAIL(h, "dinoseg_set_resolution: dino.pos_embed has not been set");
-  const int g = resolution / 8;
-  if (g > 480) DSG_FAIL(h, "resolution %d too large (patch grid %d > 480)", resolution, g);
+  const int gh = height / 8, gw = width / 8;
+  if (gh > 480 || gw > 480) DSG_FAIL(h, "resolution %dx%d too large (patch grid %dx%d, a side > 480)", height, width, gh, gw);
   const int D = h->cfg.embed_dim;
-  const size_t need = size_t(g * g + 1) * D;
+  const size_t need = size_t(gh * gw + 1) * D;
   DSG_CUDA(h, cudaSetDevice(h->device));
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   if (need > h->pos_cap) {
@@ -950,19 +961,21 @@ int dinoseg_set_resolution(dinoseg_t* h, int resolution, void* stream) {
     DSG_CUDA(h, cudaMalloc(&h->pos, need * sizeof(float)));
     h->pos_cap = need;
   }
-  DSG_CUDA(h, launch_posembed(h->pos_src, h->pos, h->cfg.pos_grid, g, D, s));
-  h->res = resolution;
-  h->g = g;
-  h->P = g * g;
-  h->Ntok = g * g + 1;
-  h->p_rep = 480 / g;  // reference pl_torch_modules.py:297
+  DSG_CUDA(h, launch_posembed(h->pos_src, h->pos, h->cfg.pos_grid, gh, gw, D, s));
+  h->res_h = height;
+  h->res_w = width;
+  h->gh = gh;
+  h->gw = gw;
+  h->P = gh * gw;
+  h->Ntok = gh * gw + 1;
+  h->p_rep = gh == gw ? 480 / gh : 0;  // reference pl_torch_modules.py:297 (predict's np.kron assumes a square grid)
   h->user.base = nullptr;  // tensor maps depend on Ntok
   for (HostLane& l : h->lanes) l.bufs.base = nullptr;
   return 0;
 }
 
 size_t dinoseg_workspace_bytes(const dinoseg_t* h, int batch) {
-  if (!h || h->res == 0 || batch <= 0) return 0;
+  if (!h || h->res_h == 0 || batch <= 0) return 0;
   return ws_layout(h, batch).total;
 }
 
@@ -1101,7 +1114,7 @@ cudaError_t launch_head_fused(dinoseg_t* h, const float* x, int M, float* logpro
   p.M = M; p.x = x; p.ln_eps = h->cfg.ln_eps;
   p.b1f = h->h1f_b; p.b2 = h->b2; p.w3 = h->w3; p.b3 = h->b3;
   p.H1 = h->cfg.head_h1; p.H2 = h->cfg.head_h2; p.C = h->cfg.n_classes;
-  p.Ntok = h->Ntok; p.g = h->g; p.p = h->p_rep;
+  p.Ntok = h->Ntok; p.gh = h->gh; p.gw = h->gw; p.p = h->p_rep;
   p.logprobs = logprobs; p.lowres = lowres; p.labels = labels;
   p.hb = g_heartbeat;
   const int m_blocks = (M + HEAD_BM - 1) / HEAD_BM;
@@ -1125,7 +1138,10 @@ struct FeatureReq {
 static int forward_impl(dinoseg_t* h, WorkBufs& w, const float* frames, const uint8_t* frames_u8, const PreprocParams* pp,
                         int batch, float* logprobs, uint8_t* lowres, int64_t* labels, cudaStream_t s,
                         const FeatureReq* feat = nullptr) {
-  if (h->res == 0) DSG_FAIL(h, "dinoseg_forward: call dinoseg_set_resolution first");
+  if (h->res_h == 0) DSG_FAIL(h, "dinoseg_forward: call dinoseg_set_resolution first");
+  if (labels && h->gh != h->gw)
+    DSG_FAIL(h, "dinoseg_forward: label maps exist for square patch grids only (resolution %dx%d); pass labels = NULL",
+             h->res_h, h->res_w);
   if (dinoseg_missing_weights(h) != 0) {
     std::string miss;
     for (auto& kv : h->slots)
@@ -1155,8 +1171,8 @@ static int forward_impl(dinoseg_t* h, WorkBufs& w, const float* frames, const ui
   };
   {
     LaunchScope ls(h, K_IM2COL, s);
-    if (frames) DSG_CUDA(h, launch_im2col(frames, w.hid, batch, h->g, s));
-    else DSG_CUDA(h, launch_im2col_u8(frames_u8, w.hid, batch, h->g, *pp, s));
+    if (frames) DSG_CUDA(h, launch_im2col(frames, w.hid, batch, h->gh, h->gw, s));
+    else DSG_CUDA(h, launch_im2col_u8(frames_u8, w.hid, batch, h->gh, h->gw, *pp, s));
     ++n;
   }
   {
@@ -1293,10 +1309,10 @@ static int forward_impl(dinoseg_t* h, WorkBufs& w, const float* frames, const ui
     LaunchScope ls(h, K_HEAD_TAIL, s);
     if (h->cfg.n_classes <= 8)
       head_tail_kernel<true, 8><<<tail_grid, 256, 0, s>>>(w.x, kLinPitch, nullptr, nullptr, logprobs, lr, tail_labels, batch,
-                                                          h->g, h->p_rep, h->Ntok, 0, h->cfg.n_classes);
+                                                          h->gh, h->gw, h->p_rep, h->Ntok, 0, h->cfg.n_classes);
     else
       head_tail_kernel<true, 16><<<tail_grid, 256, 0, s>>>(w.x, kLinPitch, nullptr, nullptr, logprobs, lr, tail_labels, batch,
-                                                           h->g, h->p_rep, h->Ntok, 0, h->cfg.n_classes);
+                                                           h->gh, h->gw, h->p_rep, h->Ntok, 0, h->cfg.n_classes);
     DSG_CUDA(h, cudaGetLastError()); ++n;
   } else {
     {
@@ -1315,10 +1331,10 @@ static int forward_impl(dinoseg_t* h, WorkBufs& w, const float* frames, const ui
     LaunchScope ls(h, K_HEAD_TAIL, s);
     if (h->cfg.n_classes <= 8)
       head_tail_kernel<false, 8><<<tail_grid, 256, 0, s>>>(w.x, h->cfg.head_h2, h->w3, h->b3, logprobs, lr, tail_labels, batch,
-                                                           h->g, h->p_rep, h->Ntok, h->cfg.head_h2, h->cfg.n_classes);
+                                                           h->gh, h->gw, h->p_rep, h->Ntok, h->cfg.head_h2, h->cfg.n_classes);
     else
       head_tail_kernel<false, 16><<<tail_grid, 256, 0, s>>>(w.x, h->cfg.head_h2, h->w3, h->b3, logprobs, lr, tail_labels, batch,
-                                                            h->g, h->p_rep, h->Ntok, h->cfg.head_h2, h->cfg.n_classes);
+                                                            h->gh, h->gw, h->p_rep, h->Ntok, h->cfg.head_h2, h->cfg.n_classes);
     DSG_CUDA(h, cudaGetLastError()); ++n;
   }
   h->launches = n;
@@ -1328,7 +1344,7 @@ static int forward_impl(dinoseg_t* h, WorkBufs& w, const float* frames, const ui
 int dinoseg_forward(dinoseg_t* h, const float* frames, int batch, float* logprobs, uint8_t* lowres, int64_t* labels,
                     void* workspace, size_t workspace_bytes, void* stream) {
   if (!h) return -1;
-  if (h->res == 0) DSG_FAIL(h, "dinoseg_forward: call dinoseg_set_resolution first");
+  if (h->res_h == 0) DSG_FAIL(h, "dinoseg_forward: call dinoseg_set_resolution first");
   if (!frames || batch <= 0 || !workspace) DSG_FAIL(h, "dinoseg_forward: bad arguments");
   DSG_CUDA(h, cudaSetDevice(h->device));
   if (bind_workspace(h, h->user, workspace, workspace_bytes, batch) != 0) return -1;
@@ -1427,7 +1443,9 @@ static int64_t predict_host_submit_impl(dinoseg_t* h, const void* host_frames, c
                                         uint8_t* host_lowres, int64_t* host_labels, void* stream, const char* who,
                                         bool streaming) {
   if (!h) return -1;
-  if (h->res == 0) DSG_FAIL(h, "%s: call dinoseg_set_resolution first", who);
+  if (h->res_h == 0) DSG_FAIL(h, "%s: call dinoseg_set_resolution first", who);
+  if (h->gh != h->gw)   // frame and label-map sizes below are those of a square grid (predict's semantics)
+    DSG_FAIL(h, "%s: the host entry points take square resolutions only (resolution %dx%d)", who, h->res_h, h->res_w);
   if (!host_frames || batch <= 0) DSG_FAIL(h, "%s: bad arguments", who);
   dinoseg::Ticket* tk = find_ticket(h, 0);
   if (!tk) DSG_FAIL(h, "%s: %d submissions are outstanding; call dinoseg_predict_host_wait first", who, dinoseg::kTickets);
@@ -1439,8 +1457,8 @@ static int64_t predict_host_submit_impl(dinoseg_t* h, const void* host_frames, c
   // submissions queue behind each other on the same three streams: the first H2D copy of submission k+1 overlaps the
   // last kernels and the last D2H copy of submission k.
   const int chunk = pick_host_chunk(h, batch, streaming);
-  const size_t frame_bytes = pp ? size_t(pp->src_h) * pp->src_w * 3 : size_t(3) * h->res * h->res * sizeof(float);
-  const size_t W = size_t(h->g) * h->p_rep;
+  const size_t frame_bytes = pp ? size_t(pp->src_h) * pp->src_w * 3 : size_t(3) * h->res_h * h->res_h * sizeof(float);
+  const size_t W = size_t(h->gh) * h->p_rep;
   const size_t label_elems = W * W;
   const size_t wbytes = dinoseg_workspace_bytes(h, chunk);
   if (!h->host_start) DSG_CUDA(h, cudaEventCreateWithFlags(&h->host_start, cudaEventDisableTiming));
@@ -1580,7 +1598,7 @@ static int64_t predict_host_submit_impl(dinoseg_t* h, const void* host_frames, c
   tk->expand = expand;
   tk->host_lowres = host_lowres;
   tk->host_labels = host_labels;
-  tk->g = h->g;
+  tk->g = h->gh;
   tk->p_rep = h->p_rep;
   tk->id = h->next_ticket++;
   return tk->id;
@@ -1656,7 +1674,7 @@ int dinoseg_forward_u8(dinoseg_t* h, const uint8_t* frames, int batch, int src_h
                        const float* std_, float* logprobs, uint8_t* lowres, int64_t* labels, void* workspace,
                        size_t workspace_bytes, void* stream) {
   if (!h) return -1;
-  if (h->res == 0) DSG_FAIL(h, "dinoseg_forward_u8: call dinoseg_set_resolution first");
+  if (h->res_h == 0) DSG_FAIL(h, "dinoseg_forward_u8: call dinoseg_set_resolution first");
   if (!frames || batch <= 0 || !workspace) DSG_FAIL(h, "dinoseg_forward_u8: bad arguments");
   PreprocParams pp;
   if (make_preproc(h, src_h, src_w, mean, std_, &pp) != 0) return -1;
@@ -1831,7 +1849,7 @@ int dinoseg_debug_set_attn_timing(long long* dev_ptr) {
 int dinoseg_cls_attention(dinoseg_t* h, const float* frames, int batch, float* attn, void* workspace,
                           size_t workspace_bytes, void* stream) {
   if (!h) return -1;
-  if (h->res == 0) DSG_FAIL(h, "dinoseg_cls_attention: call dinoseg_set_resolution first");
+  if (h->res_h == 0) DSG_FAIL(h, "dinoseg_cls_attention: call dinoseg_set_resolution first");
   if (!frames || !attn || batch <= 0 || !workspace) DSG_FAIL(h, "dinoseg_cls_attention: bad arguments");
   if (h->cfg.n_blocks < 1) DSG_FAIL(h, "dinoseg_cls_attention: the model has no transformer block");
   DSG_CUDA(h, cudaSetDevice(h->device));
@@ -1852,7 +1870,7 @@ int dinoseg_cls_attention(dinoseg_t* h, const float* frames, int batch, float* a
 // Backbone features of the last min(n_last, n_blocks) blocks in ONE pass over the blocks (no head).
 static int features_impl(dinoseg_t* h, const float* frames, const uint8_t* frames_u8, const PreprocParams* pp, int batch,
                          int n_last, float* out, void* workspace, size_t workspace_bytes, void* stream, const char* what) {
-  if (h->res == 0) DSG_FAIL(h, "%s: call dinoseg_set_resolution first", what);
+  if (h->res_h == 0) DSG_FAIL(h, "%s: call dinoseg_set_resolution first", what);
   if ((!frames && !frames_u8) || batch <= 0 || !workspace) DSG_FAIL(h, "%s: bad arguments", what);
   if (!out) DSG_FAIL(h, "%s: out is NULL", what);
   if (n_last < 1) DSG_FAIL(h, "%s: n_last must be >= 1 (got %d)", what, n_last);
@@ -1989,11 +2007,11 @@ int dinoseg_op_layernorm_f32(const float* x, const float* gamma, const float* be
 }
 
 int dinoseg_op_posembed(const float* pos_src, float* out, int G0, int g, int D, void* stream) {
-  return launch_posembed(pos_src, out, G0, g, D, static_cast<cudaStream_t>(stream)) == cudaSuccess ? 0 : -1;
+  return launch_posembed(pos_src, out, G0, g, g, D, static_cast<cudaStream_t>(stream)) == cudaSuccess ? 0 : -1;
 }
 
 int dinoseg_op_im2col(const float* frames, void* A, int B, int g, void* stream) {
-  return launch_im2col(frames, static_cast<__nv_bfloat16*>(A), B, g, static_cast<cudaStream_t>(stream)) == cudaSuccess
+  return launch_im2col(frames, static_cast<__nv_bfloat16*>(A), B, g, g, static_cast<cudaStream_t>(stream)) == cudaSuccess
              ? 0 : -1;
 }
 

@@ -43,10 +43,10 @@ struct HeadParams {
   const float* w3;        // [C, H2]
   const float* b3;        // [C]
   int H1, H2, C;          // 200, 100, n_classes
-  int Ntok, g, p;         // tokens per frame (g*g + 1), patch grid, replication factor (480 / g)
+  int Ntok, gh, gw, p;    // tokens per frame (gh*gw + 1), patch grid (rows, columns), replication factor (480 / gh)
   float* logprobs;        // [B*P, C] or null
   uint8_t* lowres;        // [B*P] or null
-  long long* labels;      // [B, g*p, g*p] or null
+  long long* labels;      // [B, g*p, g*p] or null (square grids only: gh == gw == g)
   int* hb;                // diagnostic heartbeat (see hb_mark), may be null
 };
 
@@ -359,7 +359,7 @@ head_fused_kernel(const __grid_constant__ CUtensorMap tmW1hi, const __grid_const
     // ---------------- epilogue 2: acc2 -> relu(acc2 + b2) -> layer_3 -> log_softmax -> argmax -> outputs ----------------
     const int row = (warp & 3) * 32 + lane;
     const uint32_t acc = tmem_base + (uint32_t((warp & 3) * 32) << 16) + ACC2_COL;
-    const int P = p.g * p.g, W = p.g * p.p;
+    const int P = p.gh * p.gw, W = p.gw * p.p;
     for (int bi = 0; bi < my_blocks; ++bi) {
       mbar_wait(mma2_done, bi & 1);
       __syncwarp();                                // (rows that skip the output part below rejoin here)
@@ -412,7 +412,7 @@ head_fused_kernel(const __grid_constant__ CUtensorMap tmW1hi, const __grid_const
       const int label = argmax_first<MAXC>(z, p.C);
       if (p.lowres != nullptr) p.lowres[r_out] = uint8_t(label);
       if (p.labels != nullptr) {
-        const int i = t / p.g, j = t - i * p.g;
+        const int i = t / p.gw, j = t - i * p.gw;
         long long* blk = p.labels + (size_t(b) * W + size_t(i) * p.p) * W + size_t(j) * p.p;
         if ((p.p & 1) == 0) {
           const longlong2 v2 = make_longlong2(label, label);

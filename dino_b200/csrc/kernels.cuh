@@ -38,9 +38,9 @@ __global__ void split_weight_kernel(const float* __restrict__ w, __nv_bfloat16* 
 }
 
 // ---------------------------------------------------------------------------------------
-// Positional-embedding table for a g x g patch grid (reference vision_transformer.py:202-222):
-// row 0 = pos[0] (cls); rows 1.. = bicubic resample of the G0 x G0 source grid with torch's
-// F.interpolate(scale_factor=(g+0.1)/G0, mode='bicubic', align_corners=False) semantics:
+// Positional-embedding table for a gh x gw patch grid (reference vision_transformer.py:202-222):
+// row 0 = pos[0] (cls); rows 1 + i*gw + j = bicubic resample of the G0 x G0 source grid with torch's
+// F.interpolate(scale_factor=((gh+0.1)/G0, (gw+0.1)/G0), mode='bicubic', align_corners=False) semantics, per axis:
 //   src = rscale*(dst+0.5)-0.5 with rscale = float(1/scale_factor); taps floor(src)-1..+2 clamped
 //   to [0,G0-1]; cubic-convolution weights with A = -0.75; inner sum over x, outer over y.
 // Runs once per set_resolution(); the reference recomputes it every forward.
@@ -57,17 +57,17 @@ __device__ __forceinline__ void cubic_coeffs(float t, float (&w)[4]) {
 }
 
 __global__ void posembed_bicubic_kernel(const float* __restrict__ pos_src /*[G0*G0+1, D]*/,
-                                        float* __restrict__ out /*[g*g+1, D]*/, int G0, int g, int D,
-                                        float rscale) {
+                                        float* __restrict__ out /*[gh*gw+1, D]*/, int G0, int gh, int gw, int D,
+                                        float rscale_y, float rscale_x) {
   const size_t idx = size_t(blockIdx.x) * blockDim.x + threadIdx.x;
-  const size_t total = size_t(g * g + 1) * D;
+  const size_t total = size_t(gh * gw + 1) * D;
   if (idx >= total) return;
   const int t = int(idx / D);
   const int d = int(idx - size_t(t) * D);
   if (t == 0) { out[idx] = pos_src[d]; return; }
-  const int oy = (t - 1) / g, ox = (t - 1) - oy * g;
-  const float sy = rscale * (float(oy) + 0.5f) - 0.5f;
-  const float sx = rscale * (float(ox) + 0.5f) - 0.5f;
+  const int oy = (t - 1) / gw, ox = (t - 1) - oy * gw;
+  const float sy = rscale_y * (float(oy) + 0.5f) - 0.5f;
+  const float sx = rscale_x * (float(ox) + 0.5f) - 0.5f;
   int iy = min(int(floorf(sy)), G0 - 1);
   int ix = min(int(floorf(sx)), G0 - 1);
   const float ty = fminf(fmaxf(sy - float(iy), 0.f), 1.f);
@@ -92,7 +92,7 @@ __global__ void posembed_bicubic_kernel(const float* __restrict__ pos_src /*[G0*
 
 // ---------------------------------------------------------------------------------------
 // im2col for the 8x8/stride-8 patch-embed conv (reference vision_transformer.py:153,157):
-//   A[b*P + i*g + j][c*64 + ky*8 + kx] = frame[b][c][i*8+ky][j*8+kx]
+//   A[b*P + i*gw + j][c*64 + ky*8 + kx] = frame[b][c][i*8+ky][j*8+kx],   P = gh*gw, frames [B, 3, 8*gh, 8*gw]
 // written as the bf16x3 operand [hi | lo] (2 x 192 columns, see split_weight_kernel): the rounding of
 // the pixels / conv weights to plain bf16 is the largest single contribution to the final log-prob error.
 // One thread moves two image rows of one patch (2 x 32 B in, 2 x 32 B out).
@@ -111,25 +111,25 @@ __device__ __forceinline__ void split_pack8(const float4& a0, const float4& a1, 
 }
 
 __global__ void im2col_patch8_kernel(const float* __restrict__ frames, __nv_bfloat16* __restrict__ A, int B,
-                                     int g) {
-  const int r = g * 8;
-  const size_t total = size_t(B) * 3 * g * 4 * g;  // (b, c, i, kyp, j)
+                                     int gh, int gw) {
+  const int H = gh * 8, W = gw * 8;
+  const size_t total = size_t(B) * 3 * gh * 4 * gw;  // (b, c, i, kyp, j)
   size_t idx = size_t(blockIdx.x) * blockDim.x + threadIdx.x;
   if (idx >= total) return;
-  const int j = int(idx % g); idx /= g;
+  const int j = int(idx % gw); idx /= gw;
   const int kyp = int(idx % 4); idx /= 4;
-  const int i = int(idx % g); idx /= g;
+  const int i = int(idx % gh); idx /= gh;
   const int c = int(idx % 3);
   const int b = int(idx / 3);
-  const float* src = frames + ((size_t(b) * 3 + c) * r + (i * 8 + kyp * 2)) * r + j * 8;
+  const float* src = frames + ((size_t(b) * 3 + c) * H + (i * 8 + kyp * 2)) * W + j * 8;
   const float4 a0 = __ldg(reinterpret_cast<const float4*>(src));
   const float4 a1 = __ldg(reinterpret_cast<const float4*>(src + 4));
-  const float4 b0 = __ldg(reinterpret_cast<const float4*>(src + r));
-  const float4 b1 = __ldg(reinterpret_cast<const float4*>(src + r + 4));
+  const float4 b0 = __ldg(reinterpret_cast<const float4*>(src + W));
+  const float4 b1 = __ldg(reinterpret_cast<const float4*>(src + W + 4));
   uint4 h0, l0, h1, l1;
   split_pack8(a0, a1, h0, l0);
   split_pack8(b0, b1, h1, l1);
-  __nv_bfloat16* dst = A + (size_t(b) * g * g + size_t(i) * g + j) * IM2COL_KA + c * 64 + kyp * 16;
+  __nv_bfloat16* dst = A + (size_t(b) * gh * gw + size_t(i) * gw + j) * IM2COL_KA + c * 64 + kyp * 16;
   *reinterpret_cast<uint4*>(dst) = h0;
   *reinterpret_cast<uint4*>(dst + 8) = h1;
   *reinterpret_cast<uint4*>(dst + IM2COL_K) = l0;
@@ -138,13 +138,14 @@ __global__ void im2col_patch8_kernel(const float* __restrict__ frames, __nv_bflo
 
 // ---------------------------------------------------------------------------------------
 // Preprocessing of DINOSeg.predict fused into the im2col (reference pl_torch_modules.py:33-41, :291):
-//   uint8 HWC RGB frame [H, W, 3] -> albumentations Resize(r, r) = cv2.resize(INTER_LINEAR) ->
+//   uint8 HWC RGB frame [Hs, Ws, 3] -> albumentations Resize(H, W) = cv2.resize(INTER_LINEAR) ->
 //   Normalize: (pix - mean*255) * (1 / (std*255)) in fp32 -> CHW -> 8x8 patches (bf16x3 operand as above).
 // The resize reproduces OpenCV's 8-bit bilinear path in integer arithmetic: source coordinate
 // (d + 0.5) * src/dst - 0.5, taps clamped at the borders, 11-bit fixed-point weights
 // (INTER_RESIZE_COEF_BITS), horizontal pass in int32, vertical pass
 // ((b0 * (r0 >> 4)) >> 16) + ((b1 * (r1 >> 4)) >> 16) + 2) >> 2, i.e. the uint8 image cv2 would hand to
-// Normalize.  Same-size frames (H = W = r) pass through exactly.  One thread = 8 output pixels of one row.
+// Normalize.  Each axis has its own scale src/dst; same-size frames (Hs = H, Ws = W) pass through exactly.
+// H = 8*gh, W = 8*gw.  One thread = 8 output pixels of one row.
 // ---------------------------------------------------------------------------------------
 struct PreprocParams {
   int src_h, src_w;
@@ -171,18 +172,18 @@ __device__ __forceinline__ void cv_linear_coef(int d, double scale, int src_size
 }
 
 __global__ void im2col_u8_kernel(const uint8_t* __restrict__ frames /*[B, H, W, 3]*/, __nv_bfloat16* __restrict__ A,
-                                 int B, int g, PreprocParams pp) {
-  const int r = g * 8;
-  const size_t total = size_t(B) * 3 * r * g;      // (b, c, y, j): 8 pixels each
+                                 int B, int gh, int gw, PreprocParams pp) {
+  const int H = gh * 8, W = gw * 8;
+  const size_t total = size_t(B) * 3 * H * gw;     // (b, c, y, j): 8 pixels each
   size_t idx = size_t(blockIdx.x) * blockDim.x + threadIdx.x;
   if (idx >= total) return;
-  const int j = int(idx % g); idx /= g;
-  const int y = int(idx % r); idx /= r;
+  const int j = int(idx % gw); idx /= gw;
+  const int y = int(idx % H); idx /= H;
   const int c = int(idx % 3);
   const int b = int(idx / 3);
   const uint8_t* src = frames + size_t(b) * pp.src_h * pp.src_w * 3;
-  const bool same = pp.src_h == r && pp.src_w == r;
-  const double sy = double(pp.src_h) / double(r), sx = double(pp.src_w) / double(r);
+  const bool same = pp.src_h == H && pp.src_w == W;
+  const double sy = double(pp.src_h) / double(H), sx = double(pp.src_w) / double(W);
   int y0, y1, b0, b1;
   cv_linear_coef(y, sy, pp.src_h, false, y0, y1, b0, b1);
   float v[8];
@@ -205,7 +206,7 @@ __global__ void im2col_u8_kernel(const uint8_t* __restrict__ frames /*[B, H, W, 
   uint4 hi, lo;
   split_pack8(make_float4(v[0], v[1], v[2], v[3]), make_float4(v[4], v[5], v[6], v[7]), hi, lo);
   const int i = y >> 3, ky = y & 7;
-  __nv_bfloat16* dst = A + (size_t(b) * g * g + size_t(i) * g + j) * IM2COL_KA + c * 64 + ky * 8;
+  __nv_bfloat16* dst = A + (size_t(b) * gh * gw + size_t(i) * gw + j) * IM2COL_KA + c * 64 + ky * 8;
   *reinterpret_cast<uint4*>(dst) = hi;
   *reinterpret_cast<uint4*>(dst + IM2COL_K) = lo;
 }
@@ -446,7 +447,9 @@ __device__ __forceinline__ int argmax_first(const float (&v)[HEAD_MAX_C], int C)
 // :295, :297-298 np.kron), fp32 CUDA cores, HBM-bound (reads 400 B per patch, writes 8*p*p B per patch).
 //   LINEAR = false: in = h2 = relu(layer_2(relu(layer_1))) [B*Ntok, ld] fp32 (produced by the two tensor-core GEMMs),
 //                   z = in . W3^T + b3;   LINEAR = true: in = the 'linear' head's logits [B*Ntok, ld], z = in[:C].
-// Input rows are tokens INCLUDING the cls row of every frame; output rows drop it (reference :243).
+// Input rows are tokens INCLUDING the cls row of every frame; output rows drop it (reference :243).  The patch grid is
+// gh x gw (P = gh*gw patches per frame, row-major); the label map exists for square grids only (labels == nullptr
+// otherwise).
 // Eight lanes per patch row (four rows per warp per step): the lanes read the row as consecutive float4 (coalesced),
 // keep partial dot products for all classes, all-reduce them with three xor-shuffles, and then every lane holds the
 // row's logits.  The label is written to the low-res map and - fused, labels != nullptr - replicated into its p x p
@@ -462,7 +465,7 @@ __global__ void __launch_bounds__(256)
 head_tail_kernel(const float* __restrict__ in /*[B*Ntok, ld]*/, int ld, const float* __restrict__ w3 /*[C, H2]*/,
                  const float* __restrict__ b3 /*[C]*/, float* __restrict__ logprobs /*[B*P, C] or null*/,
                  uint8_t* __restrict__ lowres /*[B*P] or null*/, long long* __restrict__ labels /*[B, g*p, g*p] or null*/,
-                 int B, int g, int p, int Ntok, int H2, int C) {
+                 int B, int gh, int gw, int p, int Ntok, int H2, int C) {
   __shared__ float sW3[LINEAR ? 1 : MAXC * HT_MAX_H2];
   __shared__ float sB3[HEAD_MAX_C];
   if constexpr (!LINEAR) {
@@ -473,12 +476,12 @@ head_tail_kernel(const float* __restrict__ in /*[B*Ntok, ld]*/, int ld, const fl
     if (threadIdx.x < HEAD_MAX_C) sB3[threadIdx.x] = threadIdx.x < C ? b3[threadIdx.x] : 0.f;
     __syncthreads();
   }
-  const int P = g * g;
+  const int P = gh * gw;
   const int total_rows = B * P;
   const int sub = threadIdx.x & 7;                           // lane within the row's group of eight
   const int grp = (blockIdx.x * blockDim.x + threadIdx.x) >> 3;
   const int ngrp = (gridDim.x * blockDim.x) >> 3;
-  const int W = g * p;
+  const int W = gw * p;
   for (int r0 = 0; r0 < total_rows; r0 += ngrp) {            // uniform trip count: the shuffles below need full warps
     const int r = r0 + grp;
     const bool live = r < total_rows;
@@ -535,7 +538,7 @@ head_tail_kernel(const float* __restrict__ in /*[B*Ntok, ld]*/, int ld, const fl
     const int label = argmax_first<MAXC>(z, C);
     if (lowres != nullptr && sub == 0) lowres[r] = uint8_t(label);
     if (labels != nullptr) {
-      const int i = t / g, j = t - i * g;
+      const int i = t / gw, j = t - i * gw;
       long long* blk = labels + (size_t(b) * W + size_t(i) * p) * W + size_t(j) * p;
       if ((p & 1) == 0) {
         const longlong2 v = make_longlong2(label, label);

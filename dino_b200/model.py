@@ -88,13 +88,20 @@ class _Backbone(nn.Module):
     def forward(self, x):
         """VisionTransformer.forward (vision_transformer.py:237-248) for all tokens: fp32 [B,3,r,r] (normalised, on the
         model's device) -> fp32 [B, N, D], N = (r/8)^2 + 1, CLS token first, after the final norm.  Runs on the GPU
-        through DINOSeg.features; the head does not run."""
+        through DINOSeg.features; the head does not run.  Square frames only, as this method has always required
+        (non-square input raises ValueError); for [B,3,H,W] frames get_intermediate_layers(x)[-1] and
+        DINOSeg.features(x)[0] return the same tensor."""
+        h, w = _frame_hw(x)
+        if h != w:
+            raise ValueError(f"model.dino(x) takes square frames [B,3,r,r], got {tuple(x.shape)}; for non-square frames "
+                             "use model.dino.get_intermediate_layers(x)[-1] or model.features(x)[0]")
         return self._model().features(x, 1)[0]
 
     def get_intermediate_layers(self, x, n=1):
         """vision_transformer.py:282-290: list of min(n, n_blocks) fp32 [B, N, D] tensors, oldest block first, each the
-        final norm of the residual stream after one of the last n blocks (one pass over the blocks).  The last element
-        equals forward(x) bit for bit."""
+        final norm of the residual stream after one of the last n blocks (one pass over the blocks).  x: fp32 [B,3,H,W]
+        with H and W multiples of 8, N = (H/8)*(W/8) + 1 (CLS, then the patches row by row).  The last element equals
+        forward(x) bit for bit."""
         return list(self._model().features(x, n).unbind(0))
 
     def get_last_selfattention(self, x):
@@ -148,6 +155,22 @@ _tolerant_pickle = types.ModuleType("dino_b200_tolerant_pickle")
 _tolerant_pickle.Unpickler = _TolerantUnpickler
 _tolerant_pickle.load = lambda f, **kw: _TolerantUnpickler(f, **kw).load()
 _tolerant_pickle.__name__ = "pickle"
+
+
+def _frame_hw(x):
+    """(H, W) of device frames fp32 [B,3,H,W]; ValueError for any other layout."""
+    if x.dim() != 4 or x.shape[1] != 3:
+        raise ValueError(f"expected frames of shape [B,3,H,W], got {tuple(x.shape)}")
+    return int(x.shape[2]), int(x.shape[3])
+
+
+def _resolution_hw(resolution):
+    """`resolution` of the raw-frame entry points: an int r (r x r) or an (H, W) pair."""
+    if isinstance(resolution, (tuple, list)):
+        if len(resolution) != 2:
+            raise ValueError(f"resolution must be an int or an (H, W) pair, got {resolution!r}")
+        return int(resolution[0]), int(resolution[1])
+    return int(resolution), int(resolution)
 
 
 class DINOSeg(nn.Module):
@@ -322,15 +345,16 @@ class DINOSeg(nn.Module):
             self._lib_res = None
         return lib
 
-    def _ensure_resolution(self, lib, res):
-        if self._lib_res != res:
-            rc = lib.dinoseg_set_resolution(self._handle, int(res), self._stream())
+    def _ensure_resolution(self, lib, hw):
+        """hw: (H, W) in pixels."""
+        if self._lib_res != hw:
+            rc = lib.dinoseg_set_resolution_hw(self._handle, int(hw[0]), int(hw[1]), self._stream())
             if rc != 0:
                 msg = _lib.last_error(self._handle)
                 if "multiple of 8" in msg:
                     raise ValueError(msg)
                 raise RuntimeError("dinoseg_set_resolution failed: " + msg)
-            self._lib_res = res
+            self._lib_res = hw
             self._workspace = None
 
     def _ensure_workspace(self, lib, batch):
@@ -345,29 +369,42 @@ class DINOSeg(nn.Module):
     # -------------------------------------------------------------------------------------
     # inference
     # -------------------------------------------------------------------------------------
+    @staticmethod
+    def _check_labels_square(hw, want_labels):
+        if want_labels and hw[0] != hw[1]:
+            raise ValueError(f"label maps (predict's np.kron tail) exist for square frames only, got {hw[0]}x{hw[1]}; "
+                             "use the log-probs or the low-res map")
+
+    def _outputs(self, b, hw, want_logprobs, want_lowres, want_labels):
+        gh, gw = hw[0] // 8, hw[1] // 8
+        dev = self.device
+        lp = torch.empty((b * gh * gw, self.n_classes), dtype=torch.float32, device=dev) if want_logprobs else None
+        low = torch.empty((b, gh, gw), dtype=torch.uint8, device=dev) if want_lowres else None
+        lab = None
+        if want_labels:
+            p = 480 // gh
+            lab = torch.empty((b, gh * p, gh * p), dtype=torch.int64, device=dev)
+        return lp, low, lab
+
     @torch.no_grad()
     def infer(self, x, want_logprobs=True, want_lowres=False, want_labels=False):
-        """Run the hot path on device frames x: fp32 [B,3,r,r] (normalised).
+        """Run the hot path on device frames x: fp32 [B,3,H,W] (normalised, H and W multiples of 8).
 
-        Returns (logprobs [B*P,C] f32 | None, lowres [B,g,g] u8 | None, labels [B,g*p,g*p] i64 | None),
-        all device tensors; asynchronous on the current stream."""
+        Returns (logprobs [B*P,C] f32 | None, lowres [B,H/8,W/8] u8 | None, labels [B,g*p,g*p] i64 | None),
+        all device tensors; asynchronous on the current stream.  P = (H/8)*(W/8), patches row by row.  Label maps are
+        predict()'s output and exist for square frames only (g = H/8 = W/8, p = 480 // g)."""
         lib = self._ensure_handle()
-        if x.dim() != 4 or x.shape[1] != 3 or x.shape[2] != x.shape[3]:
-            raise ValueError(f"expected frames of shape [B,3,r,r], got {tuple(x.shape)}")
+        hw = _frame_hw(x)
+        self._check_labels_square(hw, want_labels)
         if x.device != self.device:
             raise ValueError(f"frames are on {x.device}, model on {self.device}")
         x = x.contiguous()
         if x.dtype != torch.float32:
             x = x.float()
-        b, res = int(x.shape[0]), int(x.shape[2])
-        self._ensure_resolution(lib, res)
+        b = int(x.shape[0])
+        self._ensure_resolution(lib, hw)
         ws = self._ensure_workspace(lib, b)
-        g = res // 8
-        p = 480 // g
-        dev = self.device
-        lp = torch.empty((b * g * g, self.n_classes), dtype=torch.float32, device=dev) if want_logprobs else None
-        low = torch.empty((b, g, g), dtype=torch.uint8, device=dev) if want_lowres else None
-        lab = torch.empty((b, g * p, g * p), dtype=torch.int64, device=dev) if want_labels else None
+        lp, low, lab = self._outputs(b, hw, want_logprobs, want_lowres, want_labels)
         rc = lib.dinoseg_forward(self._handle, x.data_ptr(), b,
                                  lp.data_ptr() if lp is not None else None,
                                  low.data_ptr() if low is not None else None,
@@ -383,11 +420,15 @@ class DINOSeg(nn.Module):
 
         x: device frames fp32 [B,3,r,r] (runs the forward) or a device uint8 low-res map [B,g,g] (e.g. from infer()).
         Returns a device int32 tensor [B, 2, n_classes]: pixels of each class with x < W/2 (index 0) and x >= W/2
-        (index 1) of the (g*p) x (g*p) output map predict() would return."""
+        (index 1) of the (g*p) x (g*p) output map predict() would return.  Square frames / maps only, like predict()."""
         lib = self._ensure_handle()
         if x.dtype == torch.uint8 and x.dim() == 3:
+            if x.shape[1] != x.shape[2]:
+                raise ValueError(f"half_counts needs a square low-res map [B,g,g], got {tuple(x.shape)}")
             low = x.contiguous()
         else:
+            if x.dim() == 4 and x.shape[2] != x.shape[3]:
+                raise ValueError(f"half_counts needs square frames [B,3,r,r] (predict's label map), got {tuple(x.shape)}")
             _, low, _ = self.infer(x, want_logprobs=False, want_lowres=True)
         b, g = int(low.shape[0]), int(low.shape[1])
         p = 480 // g
@@ -400,15 +441,15 @@ class DINOSeg(nn.Module):
 
     @torch.no_grad()
     def cls_attention(self, x):
-        """Attention of the CLS query in the last kept block: [B, H, N] fp32 (see _Backbone.get_last_selfattention)."""
+        """Attention of the CLS query in the last kept block: [B, heads, N] fp32, N = (H/8)*(W/8) + 1, for fp32 frames
+        [B,3,H,W] (see _Backbone.get_last_selfattention)."""
         lib = self._ensure_handle()
-        if x.dim() != 4 or x.shape[1] != 3 or x.shape[2] != x.shape[3]:
-            raise ValueError(f"expected frames of shape [B,3,r,r], got {tuple(x.shape)}")
+        hw = _frame_hw(x)
         x = x.to(self.device).contiguous().float()
-        b, res = int(x.shape[0]), int(x.shape[2])
-        self._ensure_resolution(lib, res)
+        b = int(x.shape[0])
+        self._ensure_resolution(lib, hw)
         ws = self._ensure_workspace(lib, b)
-        n = (res // 8) ** 2 + 1
+        n = (hw[0] // 8) * (hw[1] // 8) + 1
         heads = ARCHS[self.arch]["num_heads"]
         out = torch.empty((b, heads, n), dtype=torch.float32, device=self.device)
         rc = lib.dinoseg_cls_attention(self._handle, x.data_ptr(), b, out.data_ptr(), ws.data_ptr(), ws.numel(),
@@ -419,10 +460,10 @@ class DINOSeg(nn.Module):
     @torch.no_grad()
     def features(self, x, n=1, resolution=None):
         """Backbone features of the last n blocks in one pass (no head): a device fp32 tensor [min(n, n_blocks), B, N, D],
-        N = (r/8)^2 + 1 with the CLS token first; slice k is the final norm (dino.norm) of the residual stream after
-        block n_blocks - min(n, n_blocks) + k (vision_transformer.py:282-290).  x: device fp32 [B,3,r,r] (normalised),
-        or device uint8 [B,H,W,3] raw RGB frames resized to `resolution` (default self.resolution) and normalised as
-        in infer_u8.  Asynchronous on the current stream."""
+        N = (H/8)*(W/8) + 1 with the CLS token first, then the patches row by row; slice k is the final norm (dino.norm)
+        of the residual stream after block n_blocks - min(n, n_blocks) + k (vision_transformer.py:282-290).  x: device
+        fp32 [B,3,H,W] (normalised), or device uint8 [B,Hs,Ws,3] raw RGB frames resized to `resolution` (an int r or an
+        (H, W) pair; default self.resolution) and normalised as in infer_u8.  Asynchronous on the current stream."""
         if not isinstance(n, numbers.Integral) or n < 1:
             raise ValueError(f"n must be a positive integer, got {n!r}")
         n = int(n)
@@ -433,20 +474,19 @@ class DINOSeg(nn.Module):
         if raw:
             if x.dim() != 4 or x.shape[3] != 3:
                 raise ValueError(f"expected uint8 frames of shape [B,H,W,3], got {tuple(x.shape)}")
-            res = int(self.resolution if resolution is None else resolution)
+            hw = _resolution_hw(self.resolution if resolution is None else resolution)
         else:
-            if x.dim() != 4 or x.shape[1] != 3 or x.shape[2] != x.shape[3]:
-                raise ValueError(f"expected frames of shape [B,3,r,r], got {tuple(x.shape)}")
-            res = int(x.shape[2])
-            if resolution is not None and int(resolution) != res:
-                raise ValueError(f"resolution {resolution} given for frames of size {res}")
+            hw = _frame_hw(x)
+            if resolution is not None and _resolution_hw(resolution) != hw:
+                raise ValueError(f"resolution {resolution} given for frames of size {hw[0]}x{hw[1]}")
             x = x.float()
         x = x.contiguous()
         b = int(x.shape[0])
-        self._ensure_resolution(lib, res)
+        self._ensure_resolution(lib, hw)
         ws = self._ensure_workspace(lib, b)
         n_out = min(n, self.n_blocks)
-        out = torch.empty((n_out, b, (res // 8) ** 2 + 1, self.mlp_input_dim), dtype=torch.float32, device=self.device)
+        n_tok = (hw[0] // 8) * (hw[1] // 8) + 1
+        out = torch.empty((n_out, b, n_tok, self.mlp_input_dim), dtype=torch.float32, device=self.device)
         if raw:
             mean = (C.c_float * 3)(*IMAGENET_MEAN)
             std = (C.c_float * 3)(*IMAGENET_STD)
@@ -460,7 +500,7 @@ class DINOSeg(nn.Module):
         return out
 
     def forward(self, x):
-        """pl_torch_modules.py:239-256: [B,3,r,r] -> per-patch log-probabilities [B*P, C]."""
+        """pl_torch_modules.py:239-256: [B,3,H,W] -> per-patch log-probabilities [B*P, C], P = (H/8)*(W/8)."""
         return self.infer(x, want_logprobs=True)[0]
 
     def predict(self, x):
@@ -484,24 +524,21 @@ class DINOSeg(nn.Module):
 
     @torch.no_grad()
     def infer_u8(self, frames_u8, resolution=None, want_logprobs=True, want_lowres=False, want_labels=False):
-        """Hot path on RAW device frames: uint8 [B,H,W,3] RGB (any H, W) -> resize to `resolution`, normalise
-        (ImageNet), forward.  Returns (logprobs, lowres, labels) like infer()."""
+        """Hot path on RAW device frames: uint8 [B,Hs,Ws,3] RGB (any Hs, Ws) -> resize to `resolution` (an int r for
+        r x r, or an (H, W) pair: cv2.resize(img, (W, H)) semantics), normalise (ImageNet), forward.  Returns
+        (logprobs, lowres, labels) like infer(); labels only for a square resolution."""
         lib = self._ensure_handle()
         if frames_u8.dim() != 4 or frames_u8.shape[3] != 3 or frames_u8.dtype != torch.uint8:
             raise ValueError(f"expected uint8 frames of shape [B,H,W,3], got {tuple(frames_u8.shape)} {frames_u8.dtype}")
         if frames_u8.device != self.device:
             raise ValueError(f"frames are on {frames_u8.device}, model on {self.device}")
-        res = int(self.resolution if resolution is None else resolution)
+        hw = _resolution_hw(self.resolution if resolution is None else resolution)
+        self._check_labels_square(hw, want_labels)
         frames_u8 = frames_u8.contiguous()
         b, sh, sw = int(frames_u8.shape[0]), int(frames_u8.shape[1]), int(frames_u8.shape[2])
-        self._ensure_resolution(lib, res)
+        self._ensure_resolution(lib, hw)
         ws = self._ensure_workspace(lib, b)
-        g = res // 8
-        p = 480 // g
-        dev = self.device
-        lp = torch.empty((b * g * g, self.n_classes), dtype=torch.float32, device=dev) if want_logprobs else None
-        low = torch.empty((b, g, g), dtype=torch.uint8, device=dev) if want_lowres else None
-        lab = torch.empty((b, g * p, g * p), dtype=torch.int64, device=dev) if want_labels else None
+        lp, low, lab = self._outputs(b, hw, want_logprobs, want_lowres, want_labels)
         mean = (C.c_float * 3)(*IMAGENET_MEAN)
         std = (C.c_float * 3)(*IMAGENET_STD)
         rc = lib.dinoseg_forward_u8(self._handle, frames_u8.data_ptr(), b, sh, sw, mean, std,
@@ -531,6 +568,8 @@ class DINOSeg(nn.Module):
         lib = self._ensure_handle()
         if frames.device.type != "cpu":
             raise ValueError("expected CPU frames")
+        if isinstance(resolution, (tuple, list)):
+            raise ValueError(f"the host entry points take a square resolution (an int), got {resolution!r}")
         if frames.dtype == torch.uint8:
             if frames.dim() != 4 or frames.shape[3] != 3:
                 raise ValueError("expected CPU uint8 frames of shape [B,H,W,3]")
@@ -542,7 +581,7 @@ class DINOSeg(nn.Module):
                 raise ValueError(f"expected frames of shape [B,3,r,r], got {tuple(frames.shape)}")
             frames = frames.contiguous().float()
             b, res = int(frames.shape[0]), int(frames.shape[2])
-        self._ensure_resolution(lib, res)
+        self._ensure_resolution(lib, (res, res))
         out = self._host_out(b, res // 8, output, out)
         low_ptr = out.data_ptr() if output == "lowres" else None
         lab_ptr = out.data_ptr() if output == "labels" else None

@@ -60,17 +60,26 @@ int dinoseg_missing_weights(const dinoseg_t* h);
 
 /* Replaces DINOSeg.set_resolution (pl_torch_modules.py:270-274); also builds the cached
  * bicubic positional table (vision_transformer.py:202-222).  resolution % 8 != 0 -> error
- * "Resolution should be a multiple of 8." */
+ * "Resolution should be a multiple of 8."  Same as dinoseg_set_resolution_hw(h, resolution, resolution). */
 int dinoseg_set_resolution(dinoseg_t* h, int resolution, void* stream);
+/* Frames of height x width pixels: a (height/8) x (width/8) patch grid, tokens = CLS then the patches row by row.  The
+ * positional table is resampled per axis as the reference's interpolate_pos_encoding does for [B,3,height,width] input
+ * (scale factors ((height/8 + 0.1)/G0, (width/8 + 0.1)/G0)); it is used unchanged only for a G0 x G0 grid.  Either side
+ * <= 0 or not a multiple of 8 -> "Resolution should be a multiple of 8."; either grid side > 480 -> error.
+ * With height != width: forward, features and CLS attention work (logprobs [batch*gh*gw, C], lowres [batch, gh, gw]);
+ * int64 label maps (labels != NULL) and the host entry points (dinoseg_predict_host*) are predict()'s semantics, which
+ * exist for square grids only: they return an error and enqueue nothing. */
+int dinoseg_set_resolution_hw(dinoseg_t* h, int height, int width, void* stream);
 
 size_t dinoseg_workspace_bytes(const dinoseg_t* h, int batch);
 
 /* Replaces DINOSeg.forward (pl_torch_modules.py:239-256) + the argmax / np.kron tail of
  * DINOSeg.predict (:294-298), batched.
- *   frames   : device, fp32 [batch,3,r,r] NCHW, already normalised
- *   logprobs : device, fp32 [batch*P, C] or NULL        (forward's return value)
- *   lowres   : device, uint8 [batch, g, g] or NULL       (argmax per patch)
- *   labels   : device, int64 [batch, g*p, g*p] or NULL   (p = 480 / g; predict's return value)
+ *   frames   : device, fp32 [batch,3,H,W] NCHW, already normalised (H x W as set by dinoseg_set_resolution[_hw])
+ *   logprobs : device, fp32 [batch*P, C] or NULL        (forward's return value; P = gh*gw, gh = H/8, gw = W/8)
+ *   lowres   : device, uint8 [batch, gh, gw] or NULL     (argmax per patch)
+ *   labels   : device, int64 [batch, g*p, g*p] or NULL   (square grids only, g = gh = gw, p = 480 / g; predict's return
+ *                                                         value)
  *   workspace: device scratch of at least dinoseg_workspace_bytes(h, batch) bytes, 1024-aligned */
 int dinoseg_forward(dinoseg_t* h, const float* frames, int batch, float* logprobs, uint8_t* lowres,
                     int64_t* labels, void* workspace, size_t workspace_bytes, void* stream);
@@ -101,7 +110,9 @@ int dinoseg_predict_host_wait(dinoseg_t* h, int64_t ticket);
  * transforms of DINOSeg.predict (pl_torch_modules.py:33-41, :291: albumentations Resize(r, r) -> Normalize(mean, std)
  * -> ToTensorV2) on the GPU, fused into the patch-embed im2col: the bilinear resize reproduces cv2.resize(INTER_LINEAR)
  * on 8-bit images bit for bit (11-bit fixed-point weights, result rounded to uint8), the normalisation is
- * (pix - mean*255) * (1 / (std*255)) in fp32.  mean / std: 3 host floats each (ImageNet values in the reference). */
+ * (pix - mean*255) * (1 / (std*255)) in fp32.  mean / std: 3 host floats each (ImageNet values in the reference).
+ * The frames are resized to the H x W set by dinoseg_set_resolution[_hw] (cv2.resize(img, (W, H)), each axis with its
+ * own scale); frames of exactly H x W pass through unchanged. */
 int dinoseg_forward_u8(dinoseg_t* h, const uint8_t* frames_u8, int batch, int src_h, int src_w, const float* mean,
                        const float* std_, float* logprobs, uint8_t* lowres, int64_t* labels, void* workspace,
                        size_t workspace_bytes, void* stream);
@@ -134,15 +145,15 @@ int dinoseg_get_pair_kernels(const dinoseg_t* h);   /* bit 0: GEMMs, bit 1: fuse
 
 /* CLS-query attention of the last kept block: attn [batch, heads, N] fp32 = softmax(q_cls k^T * dh^-0.5) per head,
  * i.e. row 0 of what VisionTransformer.get_last_selfattention returns (vision_transformer.py:273-280) — the only
- * row its caller reads (visualize_attention.py:46-54).  frames: device fp32 [batch,3,r,r]. */
+ * row its caller reads (visualize_attention.py:46-54).  frames: device fp32 [batch,3,H,W]; N = gh*gw + 1. */
 int dinoseg_cls_attention(dinoseg_t* h, const float* frames, int batch, float* attn, void* workspace,
                           size_t workspace_bytes, void* stream);
 
 /* Backbone features: VisionTransformer.get_intermediate_layers(x, n_last) (vision_transformer.py:282-290) in one pass
- * over the blocks, without the head.  out: device fp32 [min(n_last, n_blocks), batch, N, D], N = (r/8)^2 + 1 (CLS
+ * over the blocks, without the head.  out: device fp32 [min(n_last, n_blocks), batch, N, D], N = gh*gw + 1 (CLS
  * token first); slice k = dino.norm (eps ln_eps) applied to the residual stream after block
  * n_blocks - min(n_last, n_blocks) + k, so the last slice is what VisionTransformer.forward returns for all tokens.
- * frames: device fp32 [batch,3,r,r] (normalised).  Workspace as for dinoseg_forward (dinoseg_workspace_bytes).
+ * frames: device fp32 [batch,3,H,W] (normalised).  Workspace as for dinoseg_forward (dinoseg_workspace_bytes).
  * n_last < 1, out == NULL, no resolution set, a model without blocks or a too small workspace: error. */
 int dinoseg_features(dinoseg_t* h, const float* frames, int batch, int n_last, float* out, void* workspace,
                      size_t workspace_bytes, void* stream);
