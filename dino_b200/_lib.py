@@ -50,6 +50,11 @@ SIGNATURES = {
                                    C.c_void_p]),
     "dinoseg_features_u8": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float),
                                       C.POINTER(C.c_float), C.c_int, C.c_void_p, C.c_void_p, C.c_size_t, C.c_void_p]),
+    "dinoseg_embeddings": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_void_p, C.c_void_p, C.c_void_p,
+                                     C.c_size_t, C.c_void_p]),
+    "dinoseg_embeddings_u8": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.POINTER(C.c_float),
+                                        C.POINTER(C.c_float), C.c_int, C.c_void_p, C.c_void_p, C.c_void_p, C.c_size_t,
+                                        C.c_void_p]),
     "dinoseg_argmax_replicate": (C.c_int, [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p,
                                            C.c_void_p, C.c_void_p]),
     "dinoseg_copy_buffer": (C.c_int64, [C.c_void_p, C.c_char_p, C.c_void_p, C.c_size_t, C.c_void_p]),

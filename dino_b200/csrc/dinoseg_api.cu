@@ -349,6 +349,35 @@ cudaError_t launch_layernorm_f32(const float* x, const float* g, const float* b,
   return cudaGetLastError();
 }
 
+// Embedding kernels (kernels.cuh): clusters of EMB_SPLIT CTAs along x
+template <typename... KArgs, typename... Args>
+cudaError_t launch_emb_cluster(void (*kern)(KArgs...), dim3 grid, cudaStream_t s, Args... args) {
+  cudaLaunchConfig_t cfg = {};
+  cfg.gridDim = grid;
+  cfg.blockDim = dim3(EMB_THREADS);
+  cfg.stream = s;
+  cudaLaunchAttribute at[1];
+  at[0].id = cudaLaunchAttributeClusterDimension;
+  at[0].val.clusterDim.x = EMB_SPLIT; at[0].val.clusterDim.y = 1; at[0].val.clusterDim.z = 1;
+  cfg.attrs = at;
+  cfg.numAttrs = 1;
+  return cudaLaunchKernelEx(&cfg, kern, static_cast<KArgs>(args)...);
+}
+
+// o [B, D] bf16 = attention output of the CLS query, xc [B, D] fp32 = CLS rows of x
+cudaError_t launch_cls_attn_out(const __nv_bfloat16* qkv, const float* x, __nv_bfloat16* o, float* xc, int B, int N,
+                                int D, int H, cudaStream_t s) {
+  return launch_emb_cluster(cls_attn_out_kernel, dim3(EMB_SPLIT, H, B), s, qkv, x, o, xc, N, D);
+}
+
+// cls [B, D] (or null) = final norm of the CLS rows, mean [B, D] = final norm averaged over the patch tokens
+cudaError_t launch_embed_pool(const float* x, const float* g, const float* b, float* cls, float* mean, int B, int Ntok,
+                              int D, float eps, cudaStream_t s) {
+  if (D == 384) return launch_emb_cluster(embed_pool_kernel<384>, dim3(EMB_SPLIT, B), s, x, g, b, cls, mean, Ntok, eps);
+  if (D == 768) return launch_emb_cluster(embed_pool_kernel<768>, dim3(EMB_SPLIT, B), s, x, g, b, cls, mean, Ntok, eps);
+  return cudaErrorInvalidValue;
+}
+
 // gh x gw patch grid (gh rows, gw columns)
 cudaError_t launch_posembed(const float* pos_src, float* out, int G0, int gh, int gw, int D, cudaStream_t s) {
   if (gh == G0 && gw == G0) {
@@ -421,6 +450,12 @@ struct WorkBufs {
   CUtensorMap tm_im2col, tm_abuf, tm_hid, tm_qkv3d;                                  // A operands / attention
   CUtensorMap tm_x_out, tm_x_patch, tm_pos_add, tm_qkv_out, tm_hid_out;              // GEMM outputs / addends
   CUtensorMap tm_qkv_a, tm_h1s_out, tm_h1s_a, tm_h2_out, tm_lin_out;                 // segmentation head
+  // CLS rows of the last block (embeddings), in regions that are dead by then: the attention / LayerNorm2 output
+  // [B, D] bf16 at the start of abuf, the residual rows [B, D] fp32 (also the gather buffer of the earlier blocks'
+  // CLS rows) and the fc1 output [B, hidden] bf16 in hid
+  float* cls_x = nullptr;
+  __nv_bfloat16* cls_hid = nullptr;
+  CUtensorMap tm_cls_a, tm_cls_x, tm_cls_hid_out, tm_cls_hid_a;
 };
 
 // predict_host pipeline lane: own stream, device staging and workspace, so that the copies of one
@@ -686,6 +721,12 @@ int bind_workspace(dinoseg* h, WorkBufs& w, void* ws, size_t ws_bytes, int batch
   ok &= make_tmap_gemm_a(&w.tm_h1s_a, w.hid, M, 1, 2 * kHeadPart);
   ok &= make_tmap_gemm_out(&w.tm_h2_out, w.x, true, h->cfg.head_h2, M, 1, h->cfg.head_h2);
   ok &= make_tmap_gemm_out(&w.tm_lin_out, w.x, true, h->cfg.n_classes, M, 1, kLinPitch);   // 'linear' head logits
+  w.cls_x = reinterpret_cast<float*>(w.hid);
+  w.cls_hid = reinterpret_cast<__nv_bfloat16*>(reinterpret_cast<uint8_t*>(w.hid) + align_up(size_t(batch) * D * 4, 1024));
+  ok &= make_tmap_gemm_a(&w.tm_cls_a, w.abuf, batch, 1, D);
+  ok &= make_tmap_gemm_out(&w.tm_cls_x, w.cls_x, true, D, batch, 1, D);
+  ok &= make_tmap_gemm_out(&w.tm_cls_hid_out, w.cls_hid, false, HID, batch, 1, HID);
+  ok &= make_tmap_gemm_a(&w.tm_cls_hid_a, w.cls_hid, batch, 1, HID);
   (void)H1;
   if (!ok) DSG_FAIL(h, "cuTensorMapEncodeTiled failed for the workspace tensor maps");
   w.base = ws;
@@ -699,10 +740,11 @@ int bind_workspace(dinoseg* h, WorkBufs& w, void* ws, size_t ws_bytes, int batch
 
 namespace {
 enum Kind { K_IM2COL = 0, K_CLS, K_GEMM_PATCH, K_LN, K_GEMM_QKV, K_ATTN, K_GEMM_PROJ, K_GEMM_FC1, K_GEMM_FC2,
-            K_GEMM_HEAD, K_HEAD_TAIL, K_REPLICATE, K_MLP_FUSED, K_HEAD_FUSED, K_COUNT };
+            K_GEMM_HEAD, K_HEAD_TAIL, K_REPLICATE, K_MLP_FUSED, K_HEAD_FUSED, K_CLS_GATHER, K_CLS_ATTN_OUT, K_EMBED_POOL,
+            K_COUNT };
 const char* const kKindNames[K_COUNT] = {"im2col", "cls_row", "gemm_patch", "layernorm", "gemm_qkv", "attention",
                                          "gemm_proj", "gemm_fc1", "gemm_fc2", "gemm_head", "head_tail", "replicate",
-                                         "mlp_fused", "head_fused"};
+                                         "mlp_fused", "head_fused", "cls_gather", "cls_attn_out", "embed_pool"};
 
 // RAII pair of events around one launch (no-op unless profiling is on)
 struct LaunchScope {
@@ -1126,11 +1168,87 @@ cudaError_t launch_head_fused(dinoseg_t* h, const float* x, int M, float* logpro
 
 // Backbone features requested from forward_impl: after every block i >= first, the final LayerNorm (dino.norm) of the
 // residual stream goes to out[i - first] (fp32 [M, D] slices); backbone_only ends the pass before the head.
+// cls_rows (embeddings): only the B CLS rows are normed, out is fp32 [n, B, D] (or null) and patch_mean fp32 [B, D]
+// (or null).  Without patch_mean the last block runs for the CLS rows only after its qkv GEMM (see forward_impl).
 struct FeatureReq {
   float* out = nullptr;
   int first = 0;
   bool backbone_only = false;
+  bool cls_rows = false;
+  float* patch_mean = nullptr;
 };
+
+// The last block for the CLS rows only (embeddings without the patch mean), after LayerNorm1 and the qkv GEMM have run
+// over all rows (the CLS query attends to every key and value).  Everything after the attention reads and writes the
+// CLS rows alone, so it runs at M = B on the compact buffers of `w`: the CLS query's attention output and the gathered
+// residual rows (one kernel), the proj GEMM, the MLP as the full-size path selects it, and the fp32 final LayerNorm
+// into `cls_out` ([B, D]).  The single row block of M = B <= 128 is fine for the CTA-pair forms: their second row block
+// lies past the end, loads zeros and stores nothing.  x (all rows) is left as the qkv GEMM found it.
+static int cls_only_tail(dinoseg_t* h, WorkBufs& w, BlockW& b, int batch, float* cls_out, cudaStream_t s, int& n) {
+  const int D = h->cfg.embed_dim, HID = h->cfg.mlp_hidden;
+  const float eps = h->cfg.ln_eps;
+  const int sms = h->num_sms;
+  auto gp = [&](int N, int K, const float* bias) {
+    GemmParams p{};
+    p.N = N; p.K = K; p.rows_per_batch = batch; p.batches = 1; p.row_off = 0; p.add_batched = 0; p.bias = bias;
+    p.col_scale = 1.f; p.scale_cols = 0;
+    return p;
+  };
+  {
+    LaunchScope ls(h, K_CLS_ATTN_OUT, s);
+    DSG_CUDA(h, launch_cls_attn_out(w.qkv, w.x, w.abuf, w.cls_x, batch, h->Ntok, D, h->cfg.num_heads, s));
+    ++n;
+  }
+  {
+    LaunchScope ls(h, K_GEMM_PROJ, s);
+    DSG_CUDA(h, launch_gemm(EPI_RESID_F32, w.tm_cls_a, b.tm_proj, w.tm_cls_x, w.tm_cls_x, gp(D, D, b.proj_b), sms, s));
+    ++n;
+  }
+  if (h->fused_mlp) {
+    MlpParams p{};
+    p.M = batch; p.x = w.cls_x; p.b1 = b.fc1_b; p.b2 = b.fc2_b;
+    if (h->fuse_ln) {
+      p.fuse_ln = 1; p.ln_eps = eps;
+    } else {
+      LaunchScope ls(h, K_LN, s); DSG_CUDA(h, launch_layernorm(w.cls_x, b.ln2_g, b.ln2_b, w.abuf, batch, D, eps, false, s)); ++n;
+    }
+    LaunchScope ls(h, K_MLP_FUSED, s);
+    if (h->mlp_pair && launch_mlp_fused(w.tm_cls_a, b.tm_fc1_h, b.tm_fc2_h, w.tm_cls_x, p, sms, true, s) != cudaSuccess) {
+      (void)cudaGetLastError();
+      h->mlp_pair = false;
+    }
+    if (!h->mlp_pair) DSG_CUDA(h, launch_mlp_fused(w.tm_cls_a, b.tm_fc1_g, b.tm_fc2_g, w.tm_cls_x, p, sms, false, s));
+    ++n;
+  } else {
+    { LaunchScope ls(h, K_LN, s); DSG_CUDA(h, launch_layernorm(w.cls_x, b.ln2_g, b.ln2_b, w.abuf, batch, D, eps, false, s)); ++n; }
+    {
+      LaunchScope ls(h, K_GEMM_FC1, s);
+      const GemmParams p = gp(HID, D, b.fc1_b);
+      if (h->gemm_pair &&
+          launch_gemm_pair<EPI_GELU_BF16>(w.tm_cls_a, b.tm_fc1_p, w.tm_cls_hid_out, w.tm_cls_hid_out, p, sms, s) != cudaSuccess) {
+        (void)cudaGetLastError();
+        h->gemm_pair = false;
+      }
+      if (!h->gemm_pair) DSG_CUDA(h, launch_gemm(EPI_GELU_BF16, w.tm_cls_a, b.tm_fc1, w.tm_cls_hid_out, w.tm_cls_hid_out, p, sms, s));
+      ++n;
+    }
+    {
+      LaunchScope ls(h, K_GEMM_FC2, s);
+      const GemmParams p = gp(D, HID, b.fc2_b);
+      if (h->gemm_pair &&
+          launch_gemm_pair<EPI_RESID_F32>(w.tm_cls_hid_a, b.tm_fc2_p, w.tm_cls_x, w.tm_cls_x, p, sms, s) != cudaSuccess) {
+        (void)cudaGetLastError();
+        h->gemm_pair = false;
+      }
+      if (!h->gemm_pair) DSG_CUDA(h, launch_gemm(EPI_RESID_F32, w.tm_cls_hid_a, b.tm_fc2, w.tm_cls_x, w.tm_cls_x, p, sms, s));
+      ++n;
+    }
+  }
+  LaunchScope ls(h, K_LN, s);
+  DSG_CUDA(h, launch_layernorm_f32(w.cls_x, h->norm_g, h->norm_b, cls_out, batch, D, eps, s));
+  ++n;
+  return 0;
+}
 
 // Launch sequence of one forward pass over `batch` frames on the buffers of `w` (already bound).
 // `frames` are normalised fp32 NCHW frames, or (frames == nullptr) `frames_u8` raw uint8 HWC frames that are resized
@@ -1213,6 +1331,10 @@ static int forward_impl(dinoseg_t* h, WorkBufs& w, const float* frames, const ui
       ++n;
     }
     if (stop == 2 + 3 * i) { h->launches = n; return 0; }
+    if (feat && feat->cls_rows && !feat->patch_mean && i == h->cfg.n_blocks - 1) {
+      if (cls_only_tail(h, w, b, batch, feat->out + size_t(i - feat->first) * batch * D, s, n) != 0) return -1;
+      break;
+    }
     {
       AttnParams p{};
       p.B = batch; p.H = H; p.N = h->Ntok; p.D = D; p.out = w.abuf;
@@ -1272,7 +1394,24 @@ static int forward_impl(dinoseg_t* h, WorkBufs& w, const float* frames, const ui
         ++n;
       }
     }
-    if (feat && i >= feat->first) {
+    if (feat && feat->cls_rows && i == h->cfg.n_blocks - 1 && feat->patch_mean) {
+      LaunchScope ls(h, K_EMBED_POOL, s);
+      float* cls = feat->out ? feat->out + size_t(i - feat->first) * batch * D : nullptr;
+      DSG_CUDA(h, launch_embed_pool(w.x, h->norm_g, h->norm_b, cls, feat->patch_mean, batch, h->Ntok, D, eps, s));
+      ++n;
+    } else if (feat && feat->cls_rows && i >= feat->first && feat->out) {
+      // the B CLS rows, gathered into [B, D] and normed by the same fp32 LayerNorm kernel as the features
+      {
+        LaunchScope ls(h, K_CLS_GATHER, s);
+        DSG_CUDA(h, cudaMemcpy2DAsync(w.cls_x, size_t(D) * 4, w.x, size_t(h->Ntok) * D * 4, size_t(D) * 4, batch,
+                                      cudaMemcpyDeviceToDevice, s));
+        ++n;
+      }
+      LaunchScope ls(h, K_LN, s);
+      DSG_CUDA(h, launch_layernorm_f32(w.cls_x, h->norm_g, h->norm_b, feat->out + size_t(i - feat->first) * batch * D,
+                                       batch, D, eps, s));
+      ++n;
+    } else if (feat && !feat->cls_rows && i >= feat->first) {
       // before anything else touches x (the kernel-chain head reuses its buffer for relu(layer_2))
       LaunchScope ls(h, K_LN, s);
       DSG_CUDA(h, launch_layernorm_f32(w.x, h->norm_g, h->norm_b, feat->out + size_t(i - feat->first) * M * D, M, D, eps, s));
@@ -1903,6 +2042,49 @@ int dinoseg_features_u8(dinoseg_t* h, const uint8_t* frames, int batch, int src_
   if (make_preproc(h, src_h, src_w, mean, std_, &pp) != 0) return -1;
   return features_impl(h, nullptr, frames, &pp, batch, n_last, out, workspace, workspace_bytes, stream,
                        "dinoseg_features_u8");
+}
+
+// Image embeddings: CLS rows of the last min(n_last, n_blocks) blocks and / or the patch-token mean of the last one, in
+// one pass over the blocks (no head).
+static int embeddings_impl(dinoseg_t* h, const float* frames, const uint8_t* frames_u8, const PreprocParams* pp, int batch,
+                           int n_last, float* cls_out, float* patch_mean, void* workspace, size_t workspace_bytes,
+                           void* stream, const char* what) {
+  if (h->res_h == 0) DSG_FAIL(h, "%s: call dinoseg_set_resolution first", what);
+  if ((!frames && !frames_u8) || batch <= 0 || !workspace) DSG_FAIL(h, "%s: bad arguments", what);
+  if (!cls_out && !patch_mean) DSG_FAIL(h, "%s: cls_out and patch_mean are both NULL", what);
+  if (n_last < 1) DSG_FAIL(h, "%s: n_last must be >= 1 (got %d)", what, n_last);
+  if (h->cfg.n_blocks < 1) DSG_FAIL(h, "%s: the model has no transformer block", what);
+  DSG_CUDA(h, cudaSetDevice(h->device));
+  if (bind_workspace(h, h->user, workspace, workspace_bytes, batch) != 0) return -1;
+  FeatureReq req;
+  req.out = cls_out;
+  req.first = h->cfg.n_blocks - std::min(n_last, h->cfg.n_blocks);
+  req.backbone_only = true;
+  req.cls_rows = true;
+  req.patch_mean = patch_mean;
+  const int saved = h->debug_stop;   // a debug stop would leave the outputs unwritten
+  h->debug_stop = 0;
+  const int rc = forward_impl(h, h->user, frames, frames_u8, pp, batch, nullptr, nullptr, nullptr,
+                              static_cast<cudaStream_t>(stream), &req);
+  h->debug_stop = saved;
+  return rc;
+}
+
+int dinoseg_embeddings(dinoseg_t* h, const float* frames, int batch, int n_last, float* cls_out, float* patch_mean,
+                       void* workspace, size_t workspace_bytes, void* stream) {
+  if (!h) return -1;
+  return embeddings_impl(h, frames, nullptr, nullptr, batch, n_last, cls_out, patch_mean, workspace, workspace_bytes,
+                         stream, "dinoseg_embeddings");
+}
+
+int dinoseg_embeddings_u8(dinoseg_t* h, const uint8_t* frames, int batch, int src_h, int src_w, const float* mean,
+                          const float* std_, int n_last, float* cls_out, float* patch_mean, void* workspace,
+                          size_t workspace_bytes, void* stream) {
+  if (!h) return -1;
+  PreprocParams pp;
+  if (make_preproc(h, src_h, src_w, mean, std_, &pp) != 0) return -1;
+  return embeddings_impl(h, nullptr, frames, &pp, batch, n_last, cls_out, patch_mean, workspace, workspace_bytes, stream,
+                         "dinoseg_embeddings_u8");
 }
 
 int dinoseg_set_fused_mlp(dinoseg_t* h, int on) {

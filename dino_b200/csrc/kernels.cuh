@@ -636,6 +636,254 @@ cls_attention_kernel(const __nv_bfloat16* __restrict__ qkv, float* __restrict__ 
 }
 
 // ---------------------------------------------------------------------------------------
+// Image embeddings (DINOSeg.embeddings).  Both kernels split the tokens of a frame over a cluster of EMB_SPLIT CTAs
+// and merge the per-CTA partials in rank order through distributed shared memory: one launch, no scratch buffer, no
+// atomics.  The split does not depend on the batch size, so a frame's result is the same bits in any batch.
+// ---------------------------------------------------------------------------------------
+constexpr int EMB_SPLIT = 8;
+constexpr int EMB_THREADS = 256;
+
+__device__ __forceinline__ float ld_shared_cluster_f32(uint32_t addr) {
+  float v;
+  asm volatile("ld.shared::cluster.f32 %0, [%1];" : "=f"(v) : "r"(addr) : "memory");
+  return v;
+}
+
+// online-softmax state (running maximum m in log2 units, sum l, unnormalised output o) of one CLS-query head
+struct ClsSoftmax {
+  float m, l, o[64];
+};
+// weight of a partial with maximum pm in a merge with maximum m; a partial that has seen no key (pm = -inf) has none
+__device__ __forceinline__ float cls_softmax_scale(float pm, float m) { return pm == -INFINITY ? 0.f : exp2f(pm - m); }
+
+// Attention output of the CLS query of the last block (what the CLS row of the proj GEMM's input is):
+//   o[b, h*64 + c] = sum_j softmax_j(q_cls . k_j) v_j[c]   -> bf16 [B, D], the A operand of the proj GEMM at M = B,
+// and xc[b] = x[b*Ntok] (the CLS rows of the residual stream, fp32 [B, D]), which that GEMM adds to.
+// qkv: [B, N, 3D] bf16 as the qkv GEMM wrote it (q pre-scaled by dh^-0.5 * log2(e): scores in log2 units, as in
+// cls_attention_kernel).  Grid (EMB_SPLIT, H, B), clusters of EMB_SPLIT along x: CTA s takes the s-th contiguous chunk
+// of the keys.  Every thread keeps an online softmax over its keys: each exponent is taken against a running maximum
+// that is >= the score, so scores of any range stay finite and the result is softmax with the exact row maximum.
+// V is read as bf16 and accumulated in fp32.  Partials merge in a fixed tree: xor-butterfly in the warp, the warps in
+// order, then the CTAs in rank order.
+__global__ void __launch_bounds__(EMB_THREADS)
+cls_attn_out_kernel(const __nv_bfloat16* __restrict__ qkv, const float* __restrict__ x, __nv_bfloat16* __restrict__ o,
+                    float* __restrict__ xc, int N, int D) {
+  const int s = blockIdx.x, h = blockIdx.y, b = blockIdx.z;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const __nv_bfloat16* base = qkv + size_t(b) * N * 3 * D;
+  __shared__ float sq[64];
+  __shared__ float wm[EMB_THREADS / 32], wl[EMB_THREADS / 32], wo[EMB_THREADS / 32][64];
+  __shared__ float res[66];                                   // this CTA's (m, l, o[64])
+  if (threadIdx.x < 64) sq[threadIdx.x] = __bfloat162float(base[h * 64 + threadIdx.x]);   // token 0 = cls, q part
+  if (s == 0 && h == 0)
+    for (int d = threadIdx.x; d < D; d += EMB_THREADS) xc[size_t(b) * D + d] = x[size_t(b) * N * D + d];
+  __syncthreads();
+
+  const int chunk = (N + EMB_SPLIT - 1) / EMB_SPLIT;
+  const int j0 = s * chunk, j1 = min(N, j0 + chunk);
+  ClsSoftmax st;
+  st.m = -INFINITY; st.l = 0.f;
+#pragma unroll
+  for (int c = 0; c < 64; ++c) st.o[c] = 0.f;
+  for (int j = j0 + int(threadIdx.x); j < j1; j += EMB_THREADS) {
+    const uint4* kp = reinterpret_cast<const uint4*>(base + size_t(j) * 3 * D + D + h * 64);
+    const uint4* vp = reinterpret_cast<const uint4*>(base + size_t(j) * 3 * D + 2 * D + h * 64);
+    float sc = 0.f;
+#pragma unroll
+    for (int c = 0; c < 8; ++c) {
+      const uint4 v = __ldg(kp + c);
+      const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+      for (int e = 0; e < 4; ++e) {
+        sc = fmaf(sq[c * 8 + 2 * e], __uint_as_float(w[e] << 16), sc);
+        sc = fmaf(sq[c * 8 + 2 * e + 1], __uint_as_float(w[e] & 0xffff0000u), sc);
+      }
+    }
+    if (sc > st.m) {
+      const float a = cls_softmax_scale(st.m, sc);
+      st.l *= a;
+#pragma unroll
+      for (int c = 0; c < 64; ++c) st.o[c] *= a;
+      st.m = sc;
+    }
+    const float p = exp2f(sc - st.m);
+    st.l += p;
+#pragma unroll
+    for (int c = 0; c < 8; ++c) {
+      const uint4 v = __ldg(vp + c);
+      const uint32_t w[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+      for (int e = 0; e < 4; ++e) {
+        st.o[c * 8 + 2 * e] = fmaf(p, __uint_as_float(w[e] << 16), st.o[c * 8 + 2 * e]);
+        st.o[c * 8 + 2 * e + 1] = fmaf(p, __uint_as_float(w[e] & 0xffff0000u), st.o[c * 8 + 2 * e + 1]);
+      }
+    }
+  }
+  // warp: xor-butterfly (every lane ends with a deterministic function of the warp's 32 states; lane 0's is kept)
+#pragma unroll
+  for (int sh = 16; sh > 0; sh >>= 1) {
+    const float m2 = __shfl_xor_sync(0xffffffffu, st.m, sh), l2 = __shfl_xor_sync(0xffffffffu, st.l, sh);
+    const float m = fmaxf(st.m, m2);
+    const float sa = cls_softmax_scale(st.m, m), sb = cls_softmax_scale(m2, m);
+    st.m = m;
+    st.l = st.l * sa + l2 * sb;
+#pragma unroll
+    for (int c = 0; c < 64; ++c) st.o[c] = st.o[c] * sa + __shfl_xor_sync(0xffffffffu, st.o[c], sh) * sb;
+  }
+  if (lane == 0) {
+    wm[warp] = st.m; wl[warp] = st.l;
+#pragma unroll
+    for (int c = 0; c < 64; ++c) wo[warp][c] = st.o[c];
+  }
+  __syncthreads();
+  // CTA: the warps in order; thread c < 64 owns output column c
+  if (threadIdx.x < 64) {
+    const int c = threadIdx.x;
+    float m = -INFINITY;
+    for (int w = 0; w < EMB_THREADS / 32; ++w) m = fmaxf(m, wm[w]);
+    float l = 0.f, acc = 0.f;
+    for (int w = 0; w < EMB_THREADS / 32; ++w) {
+      const float a = cls_softmax_scale(wm[w], m);
+      l = l + wl[w] * a;
+      acc = acc + wo[w][c] * a;
+    }
+    res[2 + c] = acc;
+    if (c == 0) { res[0] = m; res[1] = l; }
+  }
+  // cluster: rank 0 merges the CTAs in rank order
+  cluster_sync_all();
+  if (s == 0 && threadIdx.x < 64) {
+    const int c = threadIdx.x;
+    float m = -INFINITY;
+    for (int r = 0; r < EMB_SPLIT; ++r) m = fmaxf(m, ld_shared_cluster_f32(mapa_rank(&res[0], r)));
+    float l = 0.f, acc = 0.f;
+    for (int r = 0; r < EMB_SPLIT; ++r) {
+      const float mr = ld_shared_cluster_f32(mapa_rank(&res[0], r));
+      const float a = cls_softmax_scale(mr, m);
+      l = l + ld_shared_cluster_f32(mapa_rank(&res[1], r)) * a;
+      acc = acc + ld_shared_cluster_f32(mapa_rank(&res[2 + c], r)) * a;
+    }
+    o[size_t(b) * D + h * 64 + c] = __float2bfloat16_rn(acc / l);
+  }
+  cluster_sync_all();                                         // the peers' shared memory stays until rank 0 has read it
+}
+
+// After the full last block: per frame, the final norm of the CLS row (cls_out [B, D], or null) and the mean of the
+// final norm over the patch tokens, patch_mean[b] = gamma * mean_t(xhat_t) + beta (xhat = (x - mean) * rstd).  The row
+// statistics and the CLS row's output use the LayerNorm kernels' arithmetic (ln384_stats / ln_out4 for D = 384, the
+// warp-per-row sums of layernorm_kernel for D = 768), so cls_out equals dino.norm's CLS row bit for bit.  x is read
+// once.  Grid (EMB_SPLIT, B), clusters of EMB_SPLIT: CTA s sums the s-th chunk of the patch tokens; per-lane sums, the
+// row groups of a warp by xor-shuffles, the warps in order, the CTAs in rank order.
+template <int D>
+__global__ void __launch_bounds__(EMB_THREADS)
+embed_pool_kernel(const float* __restrict__ x, const float* __restrict__ gamma, const float* __restrict__ beta,
+                  float* __restrict__ cls_out, float* __restrict__ patch_mean, int Ntok, float eps) {
+  static_assert(D == 384 || D == 768, "embed_pool_kernel: D = 384 or 768");
+  constexpr int NW = EMB_THREADS / 32;
+  // D = 384: eight lanes per row (four rows per warp), 12 float4 per lane; D = 768: one warp per row, 6 float4 per lane
+  constexpr int V = D == 384 ? LN384_V : D / 128;
+  constexpr int ROWS_PER_WARP = D == 384 ? 4 : 1;
+  const int s = blockIdx.x, b = blockIdx.y;
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int grp = D == 384 ? lane >> 3 : 0, sub = D == 384 ? (lane & 7) : lane;
+  constexpr int STEP = D == 384 ? 8 : 32;                     // float4 stride of a lane inside its row
+  __shared__ __align__(16) float red[NW][D];
+  __shared__ float part[D];
+  const float* xf = x + size_t(b) * Ntok * D;
+
+  auto stats = [&](const float4 (&v)[V], float& mean, float& rstd) {
+    if constexpr (D == 384) {
+      ln384_stats(v, eps, mean, rstd);
+    } else {
+      float sum = 0.f;
+#pragma unroll
+      for (int i = 0; i < V; ++i) sum += (v[i].x + v[i].y) + (v[i].z + v[i].w);
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) sum += __shfl_xor_sync(0xffffffffu, sum, o);
+      mean = sum * (1.0f / D);
+      float sq = 0.f;
+#pragma unroll
+      for (int i = 0; i < V; ++i) {
+        const float a = v[i].x - mean, bb = v[i].y - mean, c = v[i].z - mean, d = v[i].w - mean;
+        sq += (a * a + bb * bb) + (c * c + d * d);
+      }
+#pragma unroll
+      for (int o = 16; o > 0; o >>= 1) sq += __shfl_xor_sync(0xffffffffu, sq, o);
+      rstd = rsqrtf(sq * (1.0f / D) + eps);
+    }
+  };
+
+  if (s == 0 && warp == 0 && cls_out != nullptr) {
+    const float4* xr = reinterpret_cast<const float4*>(xf);
+    float4 v[V];
+#pragma unroll
+    for (int i = 0; i < V; ++i) v[i] = xr[i * STEP + sub];
+    float mean, rstd;
+    stats(v, mean, rstd);
+    if (grp == 0) {
+      float* yr = cls_out + size_t(b) * D;
+#pragma unroll
+      for (int i = 0; i < V; ++i)
+        ln_out4(yr, i * STEP + sub, v[i], mean, rstd, __ldg(reinterpret_cast<const float4*>(gamma) + i * STEP + sub),
+                __ldg(reinterpret_cast<const float4*>(beta) + i * STEP + sub));
+    }
+  }
+
+  const int P = Ntok - 1;
+  const int chunk = (P + EMB_SPLIT - 1) / EMB_SPLIT;
+  const int t0 = 1 + s * chunk, t1 = 1 + min(P, s * chunk + chunk);
+  float4 acc[V];
+#pragma unroll
+  for (int i = 0; i < V; ++i) acc[i] = make_float4(0.f, 0.f, 0.f, 0.f);
+  for (int r0 = t0; r0 < t1; r0 += NW * ROWS_PER_WARP) {      // uniform trip count: the shuffles need full warps
+    const int r = r0 + warp * ROWS_PER_WARP + grp;
+    const bool live = r < t1;
+    const float4* xr = reinterpret_cast<const float4*>(xf + size_t(live ? r : t0) * D);
+    float4 v[V];
+#pragma unroll
+    for (int i = 0; i < V; ++i) v[i] = xr[i * STEP + sub];
+    float mean, rstd;
+    stats(v, mean, rstd);
+    if (live) {
+#pragma unroll
+      for (int i = 0; i < V; ++i) {
+        acc[i].x += (v[i].x - mean) * rstd; acc[i].y += (v[i].y - mean) * rstd;
+        acc[i].z += (v[i].z - mean) * rstd; acc[i].w += (v[i].w - mean) * rstd;
+      }
+    }
+  }
+  if constexpr (D == 384) {
+#pragma unroll
+    for (int sh = 8; sh <= 16; sh <<= 1) {
+#pragma unroll
+      for (int i = 0; i < V; ++i) {
+        acc[i].x += __shfl_xor_sync(0xffffffffu, acc[i].x, sh); acc[i].y += __shfl_xor_sync(0xffffffffu, acc[i].y, sh);
+        acc[i].z += __shfl_xor_sync(0xffffffffu, acc[i].z, sh); acc[i].w += __shfl_xor_sync(0xffffffffu, acc[i].w, sh);
+      }
+    }
+  }
+  if (grp == 0) {
+#pragma unroll
+    for (int i = 0; i < V; ++i) reinterpret_cast<float4*>(red[warp])[i * STEP + sub] = acc[i];
+  }
+  __syncthreads();
+  for (int d = threadIdx.x; d < D; d += EMB_THREADS) {
+    float t = 0.f;
+    for (int w = 0; w < NW; ++w) t += red[w][d];
+    part[d] = t;
+  }
+  cluster_sync_all();
+  if (s == 0) {
+    for (int d = threadIdx.x; d < D; d += EMB_THREADS) {
+      float t = 0.f;
+      for (int r = 0; r < EMB_SPLIT; ++r) t += ld_shared_cluster_f32(mapa_rank(&part[d], r));
+      patch_mean[size_t(b) * D + d] = gamma[d] * (t / float(P)) + beta[d];
+    }
+  }
+  cluster_sync_all();
+}
+
+// ---------------------------------------------------------------------------------------
 // Nearest-neighbour block replication == np.kron(low_res, ones((p,p), int))
 // (reference pl_torch_modules.py:297-298): out[b][y][x] = low[b][y/p][x/p], int64.
 // ---------------------------------------------------------------------------------------

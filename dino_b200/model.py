@@ -457,6 +457,66 @@ class DINOSeg(nn.Module):
         self._check(rc, "dinoseg_cls_attention")
         return out
 
+    def _frames(self, x, resolution):
+        """Validated device frames of features / embeddings -> (contiguous frames, (H, W), raw)."""
+        if x.device != self.device:
+            raise ValueError(f"frames are on {x.device}, model on {self.device}")
+        raw = x.dtype == torch.uint8
+        if raw:
+            if x.dim() != 4 or x.shape[3] != 3:
+                raise ValueError(f"expected uint8 frames of shape [B,H,W,3], got {tuple(x.shape)}")
+            hw = _resolution_hw(self.resolution if resolution is None else resolution)
+        else:
+            hw = _frame_hw(x)
+            if resolution is not None and _resolution_hw(resolution) != hw:
+                raise ValueError(f"resolution {resolution} given for frames of size {hw[0]}x{hw[1]}")
+            x = x.float()
+        return x.contiguous(), hw, raw
+
+    @torch.no_grad()
+    def embeddings(self, x, n=1, avgpool=False, resolution=None):
+        """Image embeddings, one vector per frame, as upstream DINO's k-NN and linear evaluations take them: a device fp32
+        tensor, asynchronous on the current stream.  x as in features(): fp32 [B,3,H,W] or uint8 [B,Hs,Ws,3] resized to
+        `resolution`.  With L = dino.get_intermediate_layers(x, n) and n_out = min(n, n_blocks):
+
+        - avgpool=False: torch.cat([t[:, 0] for t in L], dim=-1), [B, n_out*D], oldest block first (n = 1: the CLS
+          token of model.dino(x), upstream's `model(x)` embedding).  The last block runs for the CLS row only after its
+          qkv GEMM, so its slice agrees with features() to the bf16 rounding of the attention and MLP operands; the
+          earlier slices equal features() bit for bit.
+        - avgpool=True (n_out must be 1): upstream eval_linear's
+          torch.cat((cls.unsqueeze(-1), torch.mean(L[-1][:, 1:], dim=1).unsqueeze(-1)), dim=-1).reshape(B, -1),
+          [B, 2D] with the CLS token and the patch-token mean interleaved, so that a classifier trained with upstream
+          eval_linear applies unchanged.  The last block runs in full and the CLS values equal features() bit for bit."""
+        if not isinstance(n, numbers.Integral) or n < 1:
+            raise ValueError(f"n must be a positive integer, got {n!r}")
+        n = int(n)
+        n_out = min(n, self.n_blocks)
+        if avgpool and n_out != 1:
+            raise ValueError(f"avgpool concatenates the CLS token of one block with its patch mean (upstream eval_linear "
+                             f"with n = 1); got n = {n} on a model with {self.n_blocks} blocks")
+        lib = self._ensure_handle()
+        x, hw, raw = self._frames(x, resolution)
+        b = int(x.shape[0])
+        self._ensure_resolution(lib, hw)
+        ws = self._ensure_workspace(lib, b)
+        d = self.mlp_input_dim
+        cls = torch.empty((n_out, b, d), dtype=torch.float32, device=self.device)
+        mean = torch.empty((b, d), dtype=torch.float32, device=self.device) if avgpool else None
+        mean_ptr = mean.data_ptr() if avgpool else None
+        if raw:
+            mu = (C.c_float * 3)(*IMAGENET_MEAN)
+            std = (C.c_float * 3)(*IMAGENET_STD)
+            rc = lib.dinoseg_embeddings_u8(self._handle, x.data_ptr(), b, int(x.shape[1]), int(x.shape[2]), mu, std, n,
+                                           cls.data_ptr(), mean_ptr, ws.data_ptr(), ws.numel(), self._stream())
+            self._check(rc, "dinoseg_embeddings_u8")
+        else:
+            rc = lib.dinoseg_embeddings(self._handle, x.data_ptr(), b, n, cls.data_ptr(), mean_ptr, ws.data_ptr(),
+                                        ws.numel(), self._stream())
+            self._check(rc, "dinoseg_embeddings")
+        if avgpool:
+            return torch.stack((cls[0], mean), dim=-1).reshape(b, -1)
+        return cls.permute(1, 0, 2).reshape(b, n_out * d)
+
     @torch.no_grad()
     def features(self, x, n=1, resolution=None):
         """Backbone features of the last n blocks in one pass (no head): a device fp32 tensor [min(n, n_blocks), B, N, D],

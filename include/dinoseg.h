@@ -162,6 +162,23 @@ int dinoseg_features_u8(dinoseg_t* h, const uint8_t* frames_u8, int batch, int s
                         const float* std_, int n_last, float* out, void* workspace, size_t workspace_bytes,
                         void* stream);
 
+/* Image embeddings: one vector per frame instead of the token tensor, in one pass over the blocks (no head).
+ * cls_out: device fp32 [min(n_last, n_blocks), batch, D] or NULL; slice k = dino.norm of the CLS row after block
+ * n_blocks - min(n_last, n_blocks) + k (dinoseg_features without the token axis).  patch_mean: device fp32
+ * [batch, D] or NULL = the mean over the patch tokens (not CLS) of dino.norm of the last block's output.
+ * With patch_mean == NULL the last block runs for the CLS row only after its qkv GEMM (LayerNorm1 and the qkv GEMM
+ * still cover every token); the last cls_out slice then agrees with dinoseg_features' CLS row to bf16 rounding of
+ * the attention / MLP operands, and every earlier slice is bit-identical to it.  With patch_mean, the last block
+ * runs in full and every cls_out slice is bit-identical to dinoseg_features' CLS rows.  Workspace as for
+ * dinoseg_forward.  Both outputs NULL, n_last < 1, no resolution set, a model without blocks or a too small
+ * workspace: error, nothing enqueued. */
+int dinoseg_embeddings(dinoseg_t* h, const float* frames, int batch, int n_last, float* cls_out, float* patch_mean,
+                       void* workspace, size_t workspace_bytes, void* stream);
+/* The same on raw uint8 HWC frames [batch, src_h, src_w, 3], resized and normalised as in dinoseg_forward_u8. */
+int dinoseg_embeddings_u8(dinoseg_t* h, const uint8_t* frames_u8, int batch, int src_h, int src_w, const float* mean,
+                          const float* std_, int n_last, float* cls_out, float* patch_mean, void* workspace,
+                          size_t workspace_bytes, void* stream);
+
 /* Controller-side reduction on the label map (the step after predict() in the robot pipeline, reference
  * docs/index.html "Controller": left / right obstacle masks for the potential-field controller).
  * lowres: device uint8 [batch, g, g] as written by dinoseg_forward; the output map is (g*p) x (g*p).
